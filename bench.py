@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repository's CUDA path
     python bench.py --impl reference --steps K --warmup W     # the reference algorithm on the host CPU
+    python bench.py ... --dump-outputs DIR                     # also write what the last timed step computed to DIR/*.npy
 
 Default workload: BASELINE configuration 3, the north-star target: ml::EM full-covariance GMM, N = 100M, D = 16, K = 32.
 N is FIXED: --gpus G shards the same 100M points over G GPUs ("scaling": "strong"), one process per GPU under torchrun.
@@ -46,6 +47,10 @@ DATA_SEED = 20261018
 FP64_PEAK_TFLOPS_FALLBACK = 37.0
 # CPU sample sizes of BASELINE.md §4 (upper bounds; the sample is cut to fit --cpu-budget seconds)
 CPU_SAMPLE_MAX = {"c1": 10_000, "c2": 1_000_000, "c3": 1_000_000, "c4": 200_000, "c5": 1_000_000}
+# --dump-outputs: per-point outputs are written for DUMP_BLOCKS blocks of DUMP_BLOCK_ROWS consecutive points at seeded
+# offsets; 65536 rows of K <= 64 responsibilities are at most 32 MB, within the 64 MB the files may take in all.
+DUMP_BLOCKS, DUMP_BLOCK_ROWS = 64, 1024
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def f_em(d):
@@ -56,6 +61,29 @@ def f_em(d):
 def flops_per_iteration(kind, n, d, k):
     """EM: N K F_EM(D).  K-means: N K (3D + 1) for the assignment + N (2D + 1) for the update (SURVEY.md §8d)."""
     return n * k * f_em(d) if kind == "em" else n * k * (3 * d + 1) + n * (2 * d + 1)
+
+
+def dump_sample_rows(n_total):
+    """Global indices of the points whose per-point outputs --dump-outputs writes: DUMP_BLOCKS blocks of DUMP_BLOCK_ROWS
+    consecutive points at offsets drawn from a fixed seed (the first points when there are too few for that)."""
+    import numpy as np
+    blocks = n_total // DUMP_BLOCK_ROWS
+    if blocks <= DUMP_BLOCKS:
+        return np.arange(min(n_total, DUMP_BLOCKS * DUMP_BLOCK_ROWS))
+    starts = np.sort(np.random.default_rng(DATA_SEED).choice(blocks, DUMP_BLOCKS, replace=False)) * DUMP_BLOCK_ROWS
+    return (starts[:, None] + np.arange(DUMP_BLOCK_ROWS)).ravel()
+
+
+def write_outputs(directory, arrays):
+    """Writes each entry of `arrays` (name -> array) as directory/<name>.npy in float64."""
+    import numpy as np
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs, more than the {DUMP_LIMIT_BYTES} allowed")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def parse_args():
@@ -72,7 +100,12 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-responsibilities", action="store_true", help="skip the separately declared lazy responsibilities() timing")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                                                          "(float64; per-point outputs on a fixed sample of rows) to compare two builds")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the device path (--impl b200)")
+    return args
 
 
 class ClockSampler:
@@ -401,6 +434,10 @@ def run_c1(args):
         _ = em.means, em.mixing_probabilities, em.log_likelihood
     dt = (time.perf_counter() - t0) / args.steps
     clocks.mark_end()
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"means": em.means, "covariances": [em.covariance(j) for j in range(k)],
+                                          "mixing_probabilities": em.mixing_probabilities, "log_likelihood": [em.log_likelihood],
+                                          "responsibilities": em.responsibilities, "labels": em.labels_array, "sample_rows": np.arange(n)})
     iters = em.number_iterations
     t0 = time.perf_counter()
     ref = _c1_fit_cpu(data)
@@ -440,6 +477,20 @@ class EmRunner:
     def run(self, steps, want=False):
         return self.obj.run_steps(steps, want_ll=want)
 
+    def outputs(self, rows, begin):
+        """Parameters after the last step; responsibilities and labels of the last E-step for `rows` (global indices
+        held by this rank, ascending)."""
+        np = self.np
+        means, covs, weights = self.obj.get_params()
+        resp, labels = [np.zeros((0, self.k))], [np.zeros(0, dtype=np.uint32)]
+        for run in np.split(rows, np.flatnonzero(np.diff(rows) != 1) + 1):
+            if run.size:
+                r, lab = self.obj.emit_range(int(run[0]), run.size)
+                resp.append(r)
+                labels.append(lab)
+        return {"means": means, "covariances": covs, "mixing_probabilities": weights}, \
+               {"responsibilities": np.concatenate(resp), "labels": np.concatenate(labels)}
+
 
 class KmRunner:
     """K-means through the C-ABI: a step is assignment_step + update_step (KMeans.cpp:80-109)."""
@@ -457,6 +508,10 @@ class KmRunner:
             self.obj.update()
             out.append(inertia)
         return self.np.array(out)
+
+    def outputs(self, rows, begin):
+        """Centroids after the last update; labels of the last assignment for `rows` (global indices held by this rank)."""
+        return {"centroids": self.obj.get_centroids()}, {"labels": self.obj.get_labels()[rows - begin]}
 
 
 def main():
@@ -567,6 +622,20 @@ def main():
                                   note=clock_info.get("note", "") + "; every rank sampled its own GPU, sm_mhz is the lowest median over the ranks (per_rank has each)")
     full_trace = np.concatenate([np.asarray(warm_trace, dtype=np.float64), np.asarray(trace, dtype=np.float64)])
 
+    if args.dump_outputs:
+        # the parameters are replicated on every rank; the sampled per-point outputs are gathered from the ranks holding them
+        begin, _ = cabi.shard_range(n_total, world, rank)
+        rows = dump_sample_rows(n_total)
+        rows = rows[(rows >= begin) & (rows < begin + n_local)]
+        params, points = run.outputs(rows, begin)
+        points["sample_rows"] = rows
+        if world > 1:
+            gathered = [None] * world
+            dist.all_gather_object(gathered, points)
+            points = {name: np.concatenate([g[name] for g in gathered]) for name in points}
+        if rank == 0:
+            write_outputs(args.dump_outputs, dict(params, **points, **{"log_likelihood" if kind == "em" else "inertia": trace}))
+
     # ---- e2e: the plugin call.  cppyml.clustering.EM(k).fit(X) / KMeans(k).fit(X) on a plain pageable numpy array (this
     # rank's rows), then the parameters through the Python properties.  Wall clock, max over ranks.
     e2e = None
@@ -578,6 +647,7 @@ def main():
         if world > 1:
             cppyml.distributed.init(local_rank, rank, world, uid_host)
         initialiser = cppyml.clustering.ExplicitCentroids(init_rows)
+        fit_steps = max(2, args.steps)   # the classes take no fewer than 2 maximum steps (set_maximum_steps)
 
         def one_fit():
             barrier()
@@ -587,7 +657,7 @@ def main():
                 model.set_means_initialiser(initialiser)
                 model.set_absolute_tolerance(0.0)
                 model.set_relative_tolerance(0.0)
-                model.set_maximum_steps(args.steps)
+                model.set_maximum_steps(fit_steps)
                 model.fit(host_np)
                 results = (model.means, [model.covariance(j) for j in range(k)], model.mixing_probabilities, model.log_likelihood)
                 last = model.log_likelihood
@@ -596,7 +666,7 @@ def main():
                 model = cppyml.clustering.KMeans(k)
                 model.set_centroids_initialiser(initialiser)
                 model.set_absolute_tolerance(0.0)
-                model.set_maximum_steps(args.steps)
+                model.set_maximum_steps(fit_steps)
                 model.fit(host_np)
                 results = (model.centroids, model.labels_array, model.inertia)
                 last = model.inertia
@@ -614,10 +684,10 @@ def main():
         e2e = {"value": n_total * k * iters_e2e / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": h2d / iters_e2e, "d2h_bytes_per_step": d2h / iters_e2e,
                "fit_seconds": dt, "iterations": iters_e2e,
                "what": ("cppyml.clustering.EM(K).fit(X) with X a pageable C-contiguous numpy array of this rank's rows, ExplicitCentroids start, tolerances 0, "
-                        f"maximum_steps={args.steps}; then means, covariance(k), mixing_probabilities and log_likelihood read through the Python properties"
+                        f"maximum_steps={fit_steps}; then means, covariance(k), mixing_probabilities and log_likelihood read through the Python properties"
                         if kind == "em" else
                         "cppyml.clustering.KMeans(K).fit(X) with X a pageable C-contiguous numpy array of this rank's rows, ExplicitCentroids start, tolerance 0, "
-                        f"maximum_steps={args.steps}; then centroids, labels_array (N uint32) and inertia read through the Python properties")
+                        f"maximum_steps={fit_steps}; then centroids, labels_array (N uint32) and inertia read through the Python properties")
                        + "; wall clock around the whole call sequence, max over ranks; bytes are per iteration (totals / iterations)",
                "last_scalar": last_e2e}
         if kind == "em" and iters_e2e <= len(full_trace):
