@@ -226,6 +226,11 @@ int mlb_em_force_path(mlb_em* em, int path);
 int mlb_em_conditioning(mlb_em* em, double* kappa_max, int* next_path);
 /* Number of kernels the library launched on this object since creation (bench "gpu_launches"). */
 int mlb_em_launch_count(const mlb_em* em, int64_t* launches);
+/* Diagnostic: the kernel configuration chosen for this object from (D, K, chunk), so that tests can check which template
+ * instances they run.  out[8] = {feature-space path (1 fused, 2 split, 0 none: only the direct kernels take the shape),
+ * DP, KP, NT (8-component n-tiles of a group), MW (split M kernel: feature tiles per warp; 0 off the split path),
+ * direct-kernel DP, direct-kernel NB (= DP / 8), points per chunk}.  Computes nothing. */
+int mlb_em_kernel_config(const mlb_em* em, int out[8]);
 
 /* ---------------------------------------------------------------- K-means (ML/KMeans.cpp) */
 
@@ -258,6 +263,10 @@ int mlb_km_predict(mlb_km* km, const double* x, int64_t m, int64_t ld_x, unsigne
 /* labels_ of the last assignment; rank contexts receive their own range. */
 int mlb_km_get_labels(mlb_km* km, unsigned int* labels);
 int mlb_km_launch_count(const mlb_km* km, int64_t* launches);
+/* Diagnostic: the kernel configuration chosen for this object.  out[8] = {DP, KP, KB (centroids per block), number of
+ * centroid blocks, warps per CTA of the assignment kernel, exact (1: D > 64, the reference's scan), statistics kernel
+ * (0 one-hot for K <= 32, 1 counting sort, 2 owner warps), points per chunk}.  Computes nothing. */
+int mlb_km_kernel_config(const mlb_km* km, int out[8]);
 /* As mlb_em_set_kernel_timing / mlb_em_kernel_time_ms, for the assignment kernel. */
 int mlb_km_set_kernel_timing(mlb_km* km, int enabled);
 int mlb_km_kernel_time_ms(mlb_km* km, double* total_ms, int64_t* launches);

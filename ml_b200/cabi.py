@@ -73,6 +73,7 @@ SIGNATURES = {
     "mlb_em_force_path": (ctypes.c_int, [_vp, ctypes.c_int]),
     "mlb_em_conditioning": (ctypes.c_int, [_vp, _c_dp, _c_ip]),
     "mlb_em_launch_count": (ctypes.c_int, [_vp, _c_i64p]),
+    "mlb_em_kernel_config": (ctypes.c_int, [_vp, _c_ip]),
     "mlb_km_create": (ctypes.c_int, [_vp, _vp, ctypes.c_int, ctypes.POINTER(_vp)]),
     "mlb_km_destroy": (ctypes.c_int, [_vp]),
     "mlb_km_set_centroids": (ctypes.c_int, [_vp, _vp]),
@@ -82,6 +83,7 @@ SIGNATURES = {
     "mlb_km_predict": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, ctypes.c_int64, _vp, _vp]),
     "mlb_km_get_labels": (ctypes.c_int, [_vp, _vp]),
     "mlb_km_launch_count": (ctypes.c_int, [_vp, _c_i64p]),
+    "mlb_km_kernel_config": (ctypes.c_int, [_vp, _c_ip]),
     "mlb_km_set_kernel_timing": (ctypes.c_int, [_vp, ctypes.c_int]),
     "mlb_km_kernel_time_ms": (ctypes.c_int, [_vp, _c_dp, _c_i64p]),
     "mlb_kms_supported": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int]),
@@ -126,6 +128,16 @@ def check(rc):
 
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(_vp)
+
+
+def _kernel_config(fn, handle, names):
+    out = (ctypes.c_int * 8)()
+    check(fn(handle, out))
+    return dict(zip(names, out))
+
+
+EM_CONFIG_FIELDS = ("path", "DP", "KP", "NT", "MW", "direct_DP", "direct_NB", "chunk")
+KM_CONFIG_FIELDS = ("DP", "KP", "KB", "nblocks", "nw", "exact", "stats", "chunk")
 
 
 def device_count():
@@ -428,6 +440,11 @@ class Em:
         check(lib().mlb_em_launch_count(self._h, ctypes.byref(c)))
         return c.value
 
+    def kernel_config(self):
+        """The kernels chosen for this shape (diagnostic): path (1 fused, 2 split, 0 direct only), DP, KP, NT, MW (split M
+        kernel, else 0), direct_DP, direct_NB, chunk (points per chunk of the data layout)."""
+        return _kernel_config(lib().mlb_em_kernel_config, self._h, EM_CONFIG_FIELDS)
+
     def close(self):
         if self._h:
             lib().mlb_em_destroy(self._h)
@@ -500,6 +517,11 @@ class Km:
         c = ctypes.c_int64()
         check(lib().mlb_km_launch_count(self._h, ctypes.byref(c)))
         return c.value
+
+    def kernel_config(self):
+        """The kernels chosen for this shape (diagnostic): DP, KP, KB, nblocks, nw (warps per assignment CTA), exact (D > 64
+        scan), stats (0 one-hot, 1 counting sort, 2 owner warps), chunk."""
+        return _kernel_config(lib().mlb_km_kernel_config, self._h, KM_CONFIG_FIELDS)
 
     def close(self):
         if self._h:

@@ -1974,4 +1974,19 @@ int mlb_em_launch_count(const mlb_em* em, int64_t* launches)
     return MLB_OK;
 }
 
+int mlb_em_kernel_config(const mlb_em* em, int out[8])
+{
+    MLB_ENTER(em ? em->ctx : nullptr);
+    MLB_REQUIRE(em && out, "mlb_em_kernel_config: null argument");
+    out[0] = em->path;
+    out[1] = em->DP;
+    out[2] = em->KP;
+    out[3] = em->NT;
+    out[4] = em->path == 2 ? em->MW : 0;
+    out[5] = em->dr.DP;
+    out[6] = em->dr.NB;
+    out[7] = em->data->lay.chunk;
+    return MLB_OK;
+}
+
 }  // extern "C"

@@ -1152,6 +1152,7 @@ struct mlb_km {
     std::vector<KmGpu> gpus;
     KmKernelFn fn = nullptr, fn_compact = nullptr, fn_stats = nullptr;   // fn_compact: the assignment kernel with compact per-chunk scalars
     bool stats_small = false;
+    int stats_kind = 0;          // the statistics kernel fn_stats is: 0 one-hot (km_stats_small_kernel), 1 counting sort, 2 owner warps
     bool exact = false;          // D > 64: the reference's scan (km_assign_exact_kernel) instead of the DMMA filter
     int nw = 4;                  // warps per CTA of the assignment kernel
     size_t smem = 0, smem_stats = 0;
@@ -1278,11 +1279,13 @@ int mlb_km_create(mlb_ctx* ctx, mlb_data* data, int k, mlb_km** out)
     km->fn_compact = exact ? km_assign_exact_kernel<true> : km_kernel_for<true>(DP, nw);
     km->stats_small = nblocks == 1 && KP == kKmGroup && DP <= 32;   // K <= 32: one-hot tensor-pipe statistics (its accumulators fit the registers up to D = 32)
     km->fn_stats = km->stats_small ? km_stats_small_kernel_for(DP) : nblocks == 1 ? km_stats_kernel_for<false>(DP) : km_stats_kernel_for<true>(DP);
+    km->stats_kind = km->stats_small ? 0 : 2;
     km->smem = smem;
     km->smem_stats = smem_stats;
     if (!km->stats_small && km_stats_use_sorted(data->lay.chunk, KB)) {
         km->fn_stats = nblocks == 1 ? km_stats_sorted_kernel_for<false>(DP) : km_stats_sorted_kernel_for<true>(DP);
         km->smem_stats = km_stats_sorted_smem_bytes(DP, KB, data->lay.chunk);
+        km->stats_kind = 1;
     }
     km->gpus.resize(ctx->gpus.size());
     int rc = for_each_gpu(ctx, [&](int g, Gpu& gpu) -> int {
@@ -1532,6 +1535,21 @@ int mlb_km_launch_count(const mlb_km* km, int64_t* launches)
 {
     MLB_REQUIRE(km && launches, "mlb_km_launch_count: null argument");
     *launches = km->launches;
+    return MLB_OK;
+}
+
+int mlb_km_kernel_config(const mlb_km* km, int out[8])
+{
+    MLB_ENTER(km ? km->ctx : nullptr);
+    MLB_REQUIRE(km && out, "mlb_km_kernel_config: null argument");
+    out[0] = km->DP;
+    out[1] = km->KP;
+    out[2] = km->KB;
+    out[3] = km->nblocks;
+    out[4] = km->nw;
+    out[5] = km->exact ? 1 : 0;
+    out[6] = km->stats_kind;
+    out[7] = km->data->lay.chunk;
     return MLB_OK;
 }
 

@@ -104,6 +104,8 @@ def lib():
         _lib.mlpp_oracle_em_assign_responsibilities.argtypes = [_dp, ctypes.c_int64, ctypes.c_uint, _dp, _dp, _dp, _dp, _dp]
         _lib.mlpp_oracle_kmeans_assign_label.restype = ctypes.c_uint
         _lib.mlpp_oracle_kmeans_assign_label.argtypes = [_dp, ctypes.c_int64, ctypes.c_uint, _dp, _dp]
+        _lib.mlpp_oracle_kmeans_assign_fused.restype = None
+        _lib.mlpp_oracle_kmeans_assign_fused.argtypes = [_dp, ctypes.c_int64, ctypes.c_int64, ctypes.c_uint, _dp, _up, _dp]
         _lib.mlpp_oracle_centroids_init.restype = None
         _lib.mlpp_oracle_centroids_init.argtypes = [ctypes.c_int, _dp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64,
                                                     ctypes.c_uint, ctypes.c_uint, ctypes.c_int, _dp]
@@ -312,6 +314,19 @@ def kmeans_assign_label(centroids, x):
     sq = ctypes.c_double()
     label = lib().mlpp_oracle_kmeans_assign_label(_ptr(x), d, k, _ptr(c), ctypes.byref(sq))
     return int(label), sq.value
+
+
+def kmeans_assign_fused(centroids, x):
+    """KMeans::assign_label (strict <, lowest index wins) for the rows of `x` (m, D), each squared distance summed as a
+    chain of fused multiply-adds over the dimensions in order, as the device's exact refinement evaluates it; `centroids`
+    is (D, K).  Returns (labels (m,) uint32, squared distances (m,))."""
+    c = np.ascontiguousarray(np.asarray(centroids, dtype=np.float64).T)
+    k, d = c.shape
+    x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, d)
+    labels = np.zeros(x.shape[0], dtype=np.uint32)
+    sq = np.zeros(x.shape[0])
+    lib().mlpp_oracle_kmeans_assign_fused(_ptr(x), d, x.shape[0], k, _ptr(c), labels.ctypes.data_as(_up), _ptr(sq))
+    return labels, sq
 
 
 def centroids_init(kind, data, k, seed=None, impl="oracle"):

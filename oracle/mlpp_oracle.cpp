@@ -797,6 +797,33 @@ unsigned mlpp_oracle_kmeans_assign_label(const double* x, int64_t d, unsigned k,
     return r.first;
 }
 
+// KMeans::assign_label for m points (column-major D x m) with the distance summed as a chain of fused multiply-adds,
+// s = fma(t, t, s) over the dimensions in order: the evaluation of the device's exact refinement (kmeans.cu,
+// exact_distance), which differs from the unfused sum above in the last bits.  Same scan: strict <, lowest index wins.
+void mlpp_oracle_kmeans_assign_fused(const double* x, int64_t d, int64_t m, unsigned k, const double* centroids, unsigned* labels,
+                                     double* sq_out)
+{
+    for (int64_t i = 0; i < m; ++i) {
+        const double* xi = x + i * d;
+        double best = std::numeric_limits<double>::infinity();
+        unsigned label = 0;
+        for (unsigned c = 0; c < k; ++c) {
+            const double* cc = centroids + static_cast<int64_t>(c) * d;
+            double sq = 0;
+            for (int64_t l = 0; l < d; ++l) {
+                const double t = xi[l] - cc[l];
+                sq = std::fma(t, t, sq);
+            }
+            if (sq < best) {
+                best = sq;
+                label = c;
+            }
+        }
+        labels[i] = label;
+        sq_out[i] = best;
+    }
+}
+
 // The initialisers on their own (Clustering.cpp:16-59), for PRNG-stream parity tests of the
 // product's host classes.  `seed` as in set_seed(); a default-constructed engine if !set_seed.
 void mlpp_oracle_centroids_init(int kind, const double* data, int64_t d, int64_t n, int64_t ld, unsigned k,
