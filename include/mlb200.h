@@ -265,7 +265,7 @@ int mlb_km_get_labels(mlb_km* km, unsigned int* labels);
 int mlb_km_launch_count(const mlb_km* km, int64_t* launches);
 /* Diagnostic: the kernel configuration chosen for this object.  out[8] = {DP, KP, KB (centroids per block), number of
  * centroid blocks, warps per CTA of the assignment kernel, exact (1: D > 64, the reference's scan), statistics kernel
- * (0 one-hot for K <= 32, 1 counting sort, 2 owner warps), points per chunk}.  Computes nothing. */
+ * (0 one-hot for K <= 32, 1 counting sort), points per chunk}.  Computes nothing. */
 int mlb_km_kernel_config(const mlb_km* km, int out[8]);
 /* As mlb_em_set_kernel_timing / mlb_em_kernel_time_ms, for the assignment kernel. */
 int mlb_km_set_kernel_timing(mlb_km* km, int enabled);

@@ -520,7 +520,7 @@ class Km:
 
     def kernel_config(self):
         """The kernels chosen for this shape (diagnostic): DP, KP, KB, nblocks, nw (warps per assignment CTA), exact (D > 64
-        scan), stats (0 one-hot, 1 counting sort, 2 owner warps), chunk."""
+        scan), stats (0 one-hot, 1 counting sort), chunk."""
         return _kernel_config(lib().mlb_km_kernel_config, self._h, KM_CONFIG_FIELDS)
 
     def close(self):

@@ -121,82 +121,15 @@ static int run_copy_threads(int threads, F&& body)
     return MLB_OK;
 }
 
-// An alternative upload path, OFF unless MLB200_UPLOAD=register: the caller's own pages are pinned piece by piece
-// (cudaHostRegister) and read by the DMA engine directly, one pass over host memory instead of the bounce path's three
-// (read, write to the pinned buffer, read by the DMA engine).  Pieces end on 2 MB address boundaries so that no page is
-// pinned twice; piece i + 1 is pinned and piece i - 1 released while the DMA of piece i runs.  Measured and NOT adopted
-// as a default: pinning costs more than the copies it saves.  1.6 GB per rank from pageable numpy memory, all ranks at
-// once (tools/upload_ranks.py): 2 ranks / 24 cores: bounce 24.4 GB/s per rank, registration 14.2; 8 ranks / 32 cores:
-// bounce 7.9 GB/s per rank (63 GB/s through the host's memory system), registration 4.9-6.3
-// (profiles/upload_ranks_g2_r02t.json, upload_ranks_g8_r02u.json); one rank: 50 against 18 (profiles/h2d_paths_r02a.json).
-// Returns the number of bytes it copied; the caller sends the rest (a failed registration, e.g. memory that cannot be
-// pinned) through the bounce path.
-static bool upload_by_registration(size_t total)
-{
-    const char* env = std::getenv("MLB200_UPLOAD");
-    return env && std::strcmp(env, "register") == 0 && total >= (8u << 20);
-}
-
-static int registered_h2d(Gpu& gpu, char* out, const char* in, size_t total, size_t* copied)
-{
-    constexpr size_t kPiece = 64u << 20;
-    constexpr uintptr_t kAlign = 2u << 20;
-    *copied = 0;
-    cudaEvent_t ev[2] = {nullptr, nullptr};
-    MLB_CUDA(cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming));
-    MLB_CUDA(cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming));
-    const char* prev = nullptr;
-    int turn = 0, rc = MLB_OK;
-    size_t off = 0;
-    while (off < total) {
-        const uintptr_t a = reinterpret_cast<uintptr_t>(in + off);
-        const uintptr_t cut = (a + kPiece) / kAlign * kAlign;   // a 2 MB boundary beyond a
-        const size_t len = std::min<size_t>(total - off, cut - a);
-        if (cudaHostRegister(const_cast<char*>(in + off), len, cudaHostRegisterDefault) != cudaSuccess) {
-            cudaGetLastError();   // not fatal: the bounce path takes the rest
-            break;
-        }
-        cudaError_t e = cudaMemcpyAsync(out + off, in + off, len, cudaMemcpyHostToDevice, gpu.stream);
-        if (e == cudaSuccess) e = cudaEventRecord(ev[turn & 1], gpu.stream);
-        if (prev) {
-            cudaEventSynchronize(ev[(turn - 1) & 1]);
-            cudaHostUnregister(const_cast<char*>(prev));
-        }
-        prev = in + off;
-        if (e != cudaSuccess) { set_error("upload from registered host memory failed: %s", cudaGetErrorString(e)); rc = MLB_ECUDA; break; }
-        off += len;
-        ++turn;
-    }
-    if (prev) {
-        cudaStreamSynchronize(gpu.stream);
-        cudaHostUnregister(const_cast<char*>(prev));
-    }
-    cudaEventDestroy(ev[0]);
-    cudaEventDestroy(ev[1]);
-    *copied = off;
-    return rc;
-}
-
 int staged_h2d(Gpu& gpu, void* dst_device, const void* src, size_t rows, size_t row_bytes, size_t src_stride)
 {
-    size_t total = rows * row_bytes;
+    const size_t total = rows * row_bytes;
     if (total == 0) return MLB_OK;
     const bool contiguous = src_stride == row_bytes || rows == 1;
     if (total < (1u << 20) || is_pinned_host(src)) {
         if (contiguous) MLB_CUDA(cudaMemcpyAsync(dst_device, src, total, cudaMemcpyHostToDevice, gpu.stream));
         else MLB_CUDA(cudaMemcpy2DAsync(dst_device, row_bytes, src, src_stride, row_bytes, rows, cudaMemcpyHostToDevice, gpu.stream));
         return MLB_OK;
-    }
-    if (contiguous && upload_by_registration(total)) {
-        size_t copied = 0;
-        MLB_TRY(registered_h2d(gpu, static_cast<char*>(dst_device), static_cast<const char*>(src), total, &copied));
-        if (copied == total) return MLB_OK;
-        // the rest as one dense block through the bounce buffers
-        dst_device = static_cast<char*>(dst_device) + copied;
-        src = static_cast<const char*>(src) + copied;
-        total -= copied;
-        rows = 1;
-        row_bytes = src_stride = total;
     }
     MLB_TRY(ensure_bounce(gpu));
     const size_t pieces = (total + kBounceBytes - 1) / kBounceBytes;

@@ -21,7 +21,6 @@
 // fixed-order reduction (context.cu), no floating-point atomics anywhere.
 #include <algorithm>
 #include <cmath>
-#include <cstring>
 #include <limits>
 
 #include "em_direct.cuh"
@@ -34,15 +33,6 @@ namespace mlb {
 constexpr int kTile = 64;        // points per CTA tile
 constexpr int kEmThreads = 128;  // 4 warps
 constexpr int kLogBatch = 16;    // tiles between two log() calls of the log-likelihood partial
-
-#ifdef MLB_EM_LIBM_EXP
-#define MLB_EM_EXP(x) exp(x)
-#else
-#define MLB_EM_EXP(x) exp_nonpositive((x), etab)
-#endif
-#ifndef MLB_EM_MINB_SMALL
-#define MLB_EM_MINB_SMALL 4
-#endif
 
 // ---- compile-time shape helpers -------------------------------------------------------------
 // E-step contraction steps.  One step feeds 4 features (one per lane c = lane & 3 of a quad) of 8 points to a
@@ -120,7 +110,7 @@ __device__ __forceinline__ void load_theta_frag(const double* thE, int j, int la
 // MODE 0: fused E+M step.  MODE 1: M-step from given responsibilities.  MODE 2: E-step only,
 // writing responsibilities and labels (the "emit" pass).
 template <int DP, int KP, int MODE>
-__global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? MLB_EM_MINB_SMALL : 2) em_kernel(const EmArgs p)
+__global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 : 2) em_kernel(const EmArgs p)
 {
     constexpr int NT = KP / 8, DQ = DP / 4, NE = em_ne(DP), NM = em_nm(DP);
     constexpr int ZS = DP + 4, RS = KP + 4;
@@ -284,25 +274,17 @@ __global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? ML
                 double mxs[2], sums[2];
 #pragma unroll
                 for (int mt = 0; mt < 2; ++mt) {
-#ifdef MLB_EM_FMAX_SHIFT
-                    double mx = -INFINITY;
-#pragma unroll
-                    for (int nt = 0; nt < NT; ++nt) mx = fmax(mx, fmax(acc[mt][nt][0], acc[mt][nt][1]));
-                    mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
-                    mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
-#else
                     int mkey = lse_key(acc[mt][0][0]);
 #pragma unroll
                     for (int nt = 0; nt < NT; ++nt) mkey = max(mkey, max(lse_key(acc[mt][nt][0]), lse_key(acc[mt][nt][1])));
                     mkey = max(mkey, __shfl_xor_sync(0xffffffffu, mkey, 1));
                     mkey = max(mkey, __shfl_xor_sync(0xffffffffu, mkey, 2));
                     const double mx = lse_shift_of_key(mkey);   // within 2^-20 of the largest term (fastmath.cuh)
-#endif
                     double sum = 0.0;
 #pragma unroll
                     for (int nt = 0; nt < NT; ++nt) {
-                        acc[mt][nt][0] = MLB_EM_EXP(acc[mt][nt][0] - mx);
-                        acc[mt][nt][1] = MLB_EM_EXP(acc[mt][nt][1] - mx);
+                        acc[mt][nt][0] = exp_nonpositive(acc[mt][nt][0] - mx, etab);
+                        acc[mt][nt][1] = exp_nonpositive(acc[mt][nt][1] - mx, etab);
                         sum += acc[mt][nt][0] + acc[mt][nt][1];
                     }
                     sum += __shfl_xor_sync(0xffffffffu, sum, 1);
@@ -631,13 +613,13 @@ using EmKernelFn = void (*)(EmArgs);
 template <int MODE>
 static EmKernelFn em_kernel_for(int DP, int KP)
 {
-#define MLB_EM_CASE(D_, K_) if (DP == D_ && KP == K_) return em_kernel<D_, K_, MODE>;
-#define MLB_EM_SMALL_CASE(D_, K_) if (DP == D_ && KP == K_) return em_small_kernel<D_, K_, MODE>;
-    MLB_EM_SMALL_CASE(4, 8) MLB_EM_SMALL_CASE(4, 16) MLB_EM_SMALL_CASE(4, 32)
-    MLB_EM_SMALL_CASE(8, 8) MLB_EM_SMALL_CASE(8, 16) MLB_EM_SMALL_CASE(8, 32)
-    MLB_EM_CASE(16, 8) MLB_EM_CASE(16, 16) MLB_EM_CASE(16, 32)
-#undef MLB_EM_CASE
-#undef MLB_EM_SMALL_CASE
+#define EM_CASE(D_, K_) if (DP == D_ && KP == K_) return em_kernel<D_, K_, MODE>;
+#define EM_SMALL_CASE(D_, K_) if (DP == D_ && KP == K_) return em_small_kernel<D_, K_, MODE>;
+    EM_SMALL_CASE(4, 8) EM_SMALL_CASE(4, 16) EM_SMALL_CASE(4, 32)
+    EM_SMALL_CASE(8, 8) EM_SMALL_CASE(8, 16) EM_SMALL_CASE(8, 32)
+    EM_CASE(16, 8) EM_CASE(16, 16) EM_CASE(16, 32)
+#undef EM_CASE
+#undef EM_SMALL_CASE
     return nullptr;
 }
 
@@ -1343,8 +1325,6 @@ int mlb_em_create(mlb_ctx* ctx, mlb_data* data, int k, mlb_em** out)
     em->ctx = ctx; em->data = data; em->d = data->d; em->k = k;
     em->path = fused ? 1 : split ? 2 : 0;   // 0: only the direct kernels take this shape (D > 64 or K > 256)
     em->route = em->path ? em->path : 3;
-    if (const char* env = std::getenv("MLB200_EM_PATH"))   // developer override: "direct" forces the direct kernels
-        if (std::strcmp(env, "direct") == 0) em->forced_path = 3;
     if (em->path) {
         em->DP = DP; em->KP = KP; em->NT = NT; em->NE = em_ne(DP); em->NM = em_nm(DP); em->SV = em_sv(DP, KP);
     }

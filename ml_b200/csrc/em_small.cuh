@@ -16,20 +16,11 @@
 constexpr int kSmallSub = 16;   // points per warp sub-tile
 // Warps per CTA.  Every warp is self-contained (own sub-tiles, own feature table, own accumulators), so the number is free;
 // what it sets is how many warps share the SM's registers: 4 warps x 4 CTAs at 128 registers (round 1), or 6 x 3 at 112.
-#ifndef MLB_EM_SMALL_NW
-#define MLB_EM_SMALL_NW 4
-#endif
-constexpr int kSmallWarps = MLB_EM_SMALL_NW;
+constexpr int kSmallWarps = 4;
 constexpr int kSmallThreads = kSmallWarps * 32;
-#ifndef MLB_EM_SMALL_MINB
-#define MLB_EM_SMALL_MINB 4
-#endif
 // At most 6 accumulator tiles (K <= 8, or D <= 4 with K <= 16): 96 registers suffice without spilling and a fifth
 // resident CTA per SM is worth 4-6 % (measured per 10M points: D = 8, K = 8: 0.832 -> 0.787 ms; D = 4, K = 8:
 // 0.464 -> 0.441 ms).  With 12 tiles (C2: D = 8, K = 16) the same bound spills and costs 11 % (1.337 -> 1.488 ms).
-#ifndef MLB_EM_SMALL_MINB_K8
-#define MLB_EM_SMALL_MINB_K8 5
-#endif
 
 // Slot of the constant-1 feature (weighted count): the first dead E-step slot if the packing has one (DQ odd), else a
 // new slot after the last E-step slot.
@@ -42,11 +33,7 @@ constexpr size_t em_small_smem_bytes(int DP, int KP)
 }
 
 template <int DP, int KP, int MODE>
-#ifdef MLB_EM_SMALL_MAXNREG
-__global__ void __maxnreg__(MLB_EM_SMALL_MAXNREG) em_small_kernel(const EmArgs p)
-#else
-__global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? (kSmallWarps > 4 ? 3 : 4) : ((em_small_nm(DP) * (KP / 8) <= 6) ? MLB_EM_SMALL_MINB_K8 : (em_small_nm(DP) * (KP / 8) <= 12) ? MLB_EM_SMALL_MINB : 3)) em_small_kernel(const EmArgs p)
-#endif
+__global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(DP) * (KP / 8) <= 6) ? 5 : (em_small_nm(DP) * (KP / 8) <= 12) ? 4 : 3)) em_small_kernel(const EmArgs p)
 {
     constexpr int NT = KP / 8, DQ = DP / 4, NE = em_ne(DP), NM = em_small_nm(DP);
     constexpr int RS = KP + 4, PS = NM * 8 + 4;
@@ -207,25 +194,17 @@ __global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? (kSmallWarps > 4 ? 
                 double mxs[2], sums[2];
 #pragma unroll
                 for (int mt = 0; mt < 2; ++mt) {
-#ifdef MLB_EM_FMAX_SHIFT
-                    double mx = -INFINITY;
-#pragma unroll
-                    for (int nt = 0; nt < NT; ++nt) mx = fmax(mx, fmax(acc[mt][nt][0], acc[mt][nt][1]));
-                    mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
-                    mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
-#else
                     int mkey = lse_key(acc[mt][0][0]);
 #pragma unroll
                     for (int nt = 0; nt < NT; ++nt) mkey = max(mkey, max(lse_key(acc[mt][nt][0]), lse_key(acc[mt][nt][1])));
                     mkey = max(mkey, __shfl_xor_sync(0xffffffffu, mkey, 1));
                     mkey = max(mkey, __shfl_xor_sync(0xffffffffu, mkey, 2));
                     const double mx = lse_shift_of_key(mkey);   // within 2^-20 of the largest term (fastmath.cuh)
-#endif
                     double sum = 0.0;
 #pragma unroll
                     for (int nt = 0; nt < NT; ++nt) {
-                        acc[mt][nt][0] = MLB_EM_EXP(acc[mt][nt][0] - mx);
-                        acc[mt][nt][1] = MLB_EM_EXP(acc[mt][nt][1] - mx);
+                        acc[mt][nt][0] = exp_nonpositive(acc[mt][nt][0] - mx, etab);
+                        acc[mt][nt][1] = exp_nonpositive(acc[mt][nt][1] - mx, etab);
                         sum += acc[mt][nt][0] + acc[mt][nt][1];
                     }
                     sum += __shfl_xor_sync(0xffffffffu, sum, 1);

@@ -199,7 +199,7 @@ int reduce_and_exchange_units(mlb_data* data, const std::vector<double*>& partia
 // driver thread staging through its own pinned buffer; first-touch page faults on fresh destination pages).  Large
 // copies are therefore cut into 4 MB pieces that up to four host threads pack into / unpack from pinned bounce buffers
 // (two per thread: the DMA of one piece overlaps the CPU copy of the next), so the DMA engine, not a single memcpy, is
-// the bound.  Pinned host memory (cudaMallocHost / cudaHostRegister) and small copies go straight to cudaMemcpyAsync.
+// the bound.  Pinned (page-locked) host memory and small copies go straight to cudaMemcpyAsync.
 //
 // staged_h2d: the source is `rows` rows of `row_bytes` bytes, `src_stride` bytes apart (src_stride == row_bytes: one
 // contiguous block); the destination is dense.  The DMAs are ordered on gpu.stream like any other work.  A pageable

@@ -95,19 +95,16 @@ def test_pinned_host_memory_takes_the_direct_path(cabi, ctx):
 
 
 @pytest.mark.parametrize("n,d,offset", [(3_000_000, 8, 0), (2_500_001, 16, 3), (1_100_000, 5, 1)])
-def test_upload_by_registration_round_trip(cabi, ctx, monkeypatch, n, d, offset):
-    """The opt-in upload path MLB200_UPLOAD=register (the caller's pages pinned piece by piece, read by the DMA engine
-    directly; context.cu registered_h2d): the points come back bit for bit, also from a buffer that does not start on
-    a page boundary, and the memory is an ordinary pageable array again afterwards (a second upload pins it again)."""
+def test_upload_round_trip_from_unaligned_start(cabi, ctx, n, d, offset):
+    """Large contiguous pageable uploads through the bounce buffers: the points come back bit for bit, also from a buffer
+    that does not start on a page boundary, and again on a second upload that reuses the bounce buffers."""
     rng = np.random.default_rng(n)
     backing = rng.normal(size=n * d + 8)
     points = backing[offset: offset + n * d].reshape(n, d)       # 8 * offset bytes into the allocation
-    monkeypatch.setenv("MLB200_UPLOAD", "register")
     for _ in range(2):
         dev = cabi.Data.upload(ctx, points)
         assert np.array_equal(dev.download(0, n), points)
         dev.close()
-    monkeypatch.setenv("MLB200_UPLOAD", "staged")
     dev = cabi.Data.upload(ctx, points)
     assert np.array_equal(dev.download(n - 1000, 1000), points[-1000:])
     dev.close()

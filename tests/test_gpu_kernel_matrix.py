@@ -82,7 +82,7 @@ def _em_id(case):
 
 
 # (D, K, N, chunk, env, expected (DP, KP, KB, nblocks, nw, exact, stats, chunk)); stats 0 one-hot km_stats_small_kernel,
-# 1 counting sort km_stats_sorted_kernel, 2 owner warps km_stats_kernel.  nw = warps per CTA of km_assign_kernel.
+# 1 counting sort km_stats_sorted_kernel.  nw = warps per CTA of km_assign_kernel.
 KM_SHAPES = [
     (3, 31, N_A, {}, (4, 32, 32, 1, 4, 0, 0)),
     (4, 1200, N_A, {}, (4, 1216, 1216, 1, 8, 0, 1)),
@@ -104,8 +104,8 @@ KM_SHAPES = [
     (65, 3, N_A, {}, (128, 32, 32, 1, 4, 1, 1)),
     (100, 40, N_B, {}, (128, 64, 64, 1, 4, 1, 1)),
     (8, 150, N_A, {"MLB200_KM_BLOCK": "64"}, (8, 192, 64, 3, 4, 0, 1)),
-    (8, 150, N_B, {"MLB200_KM_BLOCK": "64", "MLB200_KM_STATS": "owner"}, (8, 192, 64, 3, 4, 0, 2)),
-    (16, 100, N_A, {"MLB200_KM_STATS": "owner"}, (16, 128, 128, 1, 4, 0, 2)),
+    (8, 150, N_B, {"MLB200_KM_BLOCK": "64"}, (8, 192, 64, 3, 4, 0, 1)),
+    (16, 100, N_A, {}, (16, 128, 128, 1, 4, 0, 1)),
 ]
 KM_CASES = []
 for _d, _k, _n, _env, _cfg in KM_SHAPES:

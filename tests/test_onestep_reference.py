@@ -142,15 +142,15 @@ def test_km_step_within_1e14_of_long_double():
 
 # ---------------------------------------------------------------- coverage of the kernel matrix
 # Every instance the dispatch code can launch.  Mirrors em_kernel_for and the split / direct selection in mlb_em_create
-# (ml_b200/csrc/em.cu), and km_kernel_for, km_warps_per_cta, the statistics selection in mlb_km_create and
-# km_stats_use_sorted (ml_b200/csrc/kmeans.cu).  A new instance there belongs here and in the matrix.
+# (ml_b200/csrc/em.cu), and km_kernel_for, km_warps_per_cta and the statistics selection in mlb_km_create and
+# mlb_kms_create (ml_b200/csrc/kmeans.cu).  A new instance there belongs here and in the matrix.
 FUSED = {(dp, kp, mode) for dp in (4, 8, 16) for kp in (8, 16, 32) for mode in (0, 1, 2)}
 SPLIT = {(nt, mw) for nt in (2, 4, 8) for mw in (3, 4, 5)}
 DIRECT_NB = {1, 2, 0}                                  # em_direct_e_kernel<NB>: 1, 2, and 0 for every wider D
 KM_ASSIGN = {(dp, nw, compact) for dp, nws in ((4, (4, 8, 16)), (8, (4, 8, 16)), (16, (4, 8, 16)), (32, (4, 8, 16)), (64, (4, 8)))
              for nw in nws for compact in (False, True)}
 KM_STATS = ({("small", dp) for dp in (4, 8, 16, 32)} | {("sorted", dp, blocked) for dp in (4, 8, 16, 32, 64, 128) for blocked in (False,)}
-            | {("sorted", 8, True), ("owner", 8, True), ("owner", 16, False)} | {("exact", False), ("exact", True)})
+            | {("sorted", 8, True)} | {("exact", False), ("exact", True)})
 
 
 def test_kernel_matrix_covers_every_instance():
@@ -171,7 +171,7 @@ def test_kernel_matrix_covers_every_instance():
             stats |= {("exact", False), ("exact", True)}    # assign (full statistics) and predict (compact)
         else:
             assign |= {(dp, nw, False), (dp, nw, True)}     # assign + update, and predict
-        name = ("small", "sorted", "owner")[kind]
+        name = ("small", "sorted")[kind]
         stats.add((name, dp) if kind == 0 else (name, dp, nblocks > 1))
     assert FUSED <= fused, FUSED - fused
     assert SPLIT <= split, SPLIT - split

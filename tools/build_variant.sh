@@ -1,5 +1,5 @@
 #!/bin/bash
-# Developer tool: builds build/variants/libmlb200_<name>.so with extra nvcc flags (e.g. -DMLB_EM_LIBM_EXP) so that
+# Developer tool: builds build/variants/libmlb200_<name>.so with extra nvcc flags (e.g. -maxrregcount=96) so that
 # tools/quick_bench.py can time experimental kernels side by side (MLB200_LIB=<path> python tools/quick_bench.py ...).
 set -e
 name=$1; shift
