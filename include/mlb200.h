@@ -200,6 +200,24 @@ int mlb_em_emit_range(mlb_em* em, int64_t begin, int64_t count, double* resp_out
  * (may be NULL) is the argmax of each row (first maximum wins).  Runs on the first local GPU. */
 int mlb_em_predict(mlb_em* em, const double* x, int64_t m, int64_t ld_x, double* resp_out, int64_t ld_out, unsigned int* labels_out);
 
+/* Scoring.  l(x) = log sum_k w_k N(x | mu_k, Sigma_k) under the CURRENT parameters (after a fit: the post-fit ones,
+ * unlike the log-likelihood a step reports, which belongs to the parameters before its M-step).  l(x) includes the
+ * -D/2 log(2 pi) term and is evaluated with the E-step's log-sum-exp shift, so it stays finite where every density
+ * underflows.  Scoring takes the kernels predict takes (the direct kernels when mlb_em_conditioning reports path 3)
+ * and changes nothing a step, emit or predict reads: parameters, log-likelihoods, stored responsibilities, path and
+ * kernel timing stay as they were.  A point's value depends only on the point and the parameters.
+ *
+ * log p(x) under the current parameters for m host points (column-major D x m, stride ld_x >= D), on the first local GPU,
+ * staged like mlb_em_predict.  log_density_out (m values) and mean_out may each be NULL.  The mean is summed in a fixed
+ * order: bitwise repeatable, and independent of the staging size.  The mean of m = 0 points is NaN. */
+int mlb_em_score(mlb_em* em, const double* x, int64_t m, int64_t ld_x, double* log_density_out, double* mean_out);
+
+/* The same for the resident points of the fit, on every GPU of the context, without a new upload.  log_density_out gets
+ * n_total values, or the rank's own range in a rank context; mean_out gets the mean over ALL points.  Per-chunk sums go
+ * through the context's fixed reduction (8 virtual shards, one exchange, fixed tree), so the mean is bitwise the same for
+ * G = 1, 2, 4, 8 and for rank contexts.  Collective in rank contexts. */
+int mlb_em_score_fitted(mlb_em* em, double* log_density_out, double* mean_out);
+
 /* Per-launch device timing of the dominant kernel (the fused E+M kernel) for roofline reports:
  * CUDA events recorded on the launching stream around each launch while enabled (at most 4096
  * launches are kept).  mlb_em_kernel_time_ms synchronises and returns the summed duration and the

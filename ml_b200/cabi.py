@@ -66,6 +66,8 @@ SIGNATURES = {
     "mlb_em_emit": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, _vp]),
     "mlb_em_emit_range": (ctypes.c_int, [_vp, ctypes.c_int64, ctypes.c_int64, _vp, ctypes.c_int64, _vp]),
     "mlb_em_predict": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, ctypes.c_int64, _vp, ctypes.c_int64, _vp]),
+    "mlb_em_score": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, ctypes.c_int64, _vp, _c_dp]),
+    "mlb_em_score_fitted": (ctypes.c_int, [_vp, _vp, _c_dp]),
     "mlb_em_set_kernel_timing": (ctypes.c_int, [_vp, ctypes.c_int]),
     "mlb_em_kernel_time_ms": (ctypes.c_int, [_vp, _c_dp, _c_i64p]),
     "mlb_em_last_path": (ctypes.c_int, [_vp, _c_ip]),
@@ -359,6 +361,23 @@ class Em:
         labels = np.empty(m, dtype=np.uint32) if want_labels else None
         check(lib().mlb_em_predict(self._h, _ptr(pts), m, self.d, _ptr(resp), max(m, 1), _ptr(labels)))
         return resp, labels
+
+    def score(self, points, want_log_densities=True):
+        """log p(x) of the rows of `points` (m, D) under the current parameters, and their mean."""
+        pts = np.ascontiguousarray(points, dtype=np.float64)
+        assert pts.ndim == 2 and pts.shape[1] == self.d
+        m = pts.shape[0]
+        ll = np.empty(m) if want_log_densities else None
+        mean = ctypes.c_double()
+        check(lib().mlb_em_score(self._h, _ptr(pts), m, self.d, _ptr(ll), ctypes.byref(mean)))
+        return ll, mean.value
+
+    def score_fitted(self, want_log_densities=True):
+        """log p(x) of the resident points (n_local values) under the current parameters, and the mean over all points."""
+        ll = np.empty(self.n_local) if want_log_densities else None
+        mean = ctypes.c_double()
+        check(lib().mlb_em_score_fitted(self._h, _ptr(ll), ctypes.byref(mean)))
+        return ll, mean.value
 
     def step(self):
         ll = ctypes.c_double()

@@ -80,9 +80,10 @@ struct EmArgs {
     const double* r_in;    // MODE 1: responsibilities, column-major local rows
     long long r_ld;
     double* r_out;         // MODE 2: responsibilities of [range_begin, range_begin + range_count), column-major
+                           // MODE 3: log p(x) of the same points
     long long r_out_ld;
     unsigned* labels_out;  // MODE 2
-    long long range_begin, range_count;
+    long long range_begin, range_count;   // MODE 2 and 3
 };
 
 __device__ __forceinline__ long long min64(long long a, long long b) { return a < b ? a : b; }
@@ -108,9 +109,9 @@ __device__ __forceinline__ void load_theta_frag(const double* thE, int j, int la
 }
 
 // MODE 0: fused E+M step.  MODE 1: M-step from given responsibilities.  MODE 2: E-step only,
-// writing responsibilities and labels (the "emit" pass).
+// writing responsibilities and labels (the "emit" pass).  MODE 3: E-step only, writing log p(x) per point (scoring).
 template <int DP, int KP, int MODE>
-__global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 : 2) em_kernel(const EmArgs p)
+__global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE >= 2) ? 4 : 2) em_kernel(const EmArgs p)
 {
     constexpr int NT = KP / 8, DQ = DP / 4, NE = em_ne(DP), NM = em_nm(DP);
     constexpr int ZS = DP + 4, RS = KP + 4;
@@ -143,7 +144,7 @@ __global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 
     const int wm = warp / WN, wn = warp % WN;
     int ia[MW], ib[MW];
     double sacc[MW][NW][2];
-    if (MODE != 2) {
+    if (MODE < 2) {
 #pragma unroll
         for (int i = 0; i < MW; ++i) {
             const int mt = wm * MW + i;
@@ -177,8 +178,8 @@ __global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 
         if (tid < kTile) Z[tid * ZS + DP] = tid < nvalid ? 1.0 : 0.0;
     };
 
-    const long long work_begin = MODE == 2 ? p.range_begin : 0;
-    const long long work_end = MODE == 2 ? p.range_begin + p.range_count : p.n_local;
+    const long long work_begin = MODE >= 2 ? p.range_begin : 0;
+    const long long work_end = MODE >= 2 ? p.range_begin + p.range_count : p.n_local;
 
     for (;;) {
         __syncthreads();
@@ -190,7 +191,7 @@ __global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 
         const long long p_end = min64(p_begin + p.chunk, work_end);
         const int ntiles = static_cast<int>((p_end - p_begin + kTile - 1) / kTile);
 
-        if (MODE != 2) {
+        if (MODE < 2) {
 #pragma unroll
             for (int i = 0; i < MW; ++i)
 #pragma unroll
@@ -308,6 +309,8 @@ __global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 
 #pragma unroll
                         for (int nt = 0; nt < NT; ++nt)
                             *reinterpret_cast<double2*>(R + pl * RS + 8 * nt + 2 * c) = make_double2(acc[mt][nt][0] * inv, acc[mt][nt][1] * inv);
+                    } else if (MODE == 3) {
+                        if (c == 0 && pl < nvalid) p.r_out[(tile0 - p.range_begin) + pl] = (mxs[mt] + log(sums[mt])) - 0.5 * d * kLog2Pi;
                     } else {
                         // emit: responsibilities_ (EM.cpp:213-218) and labels_ (EM.cpp:289-304, first maximum wins)
                         double best = -1.0;
@@ -333,7 +336,7 @@ __global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 
                     }
                 }
             }
-            if (MODE != 2) {
+            if (MODE < 2) {
                 __syncthreads();
                 // ---------------- M-step: S += Phi(Z)^T . R over the tile's 64 points
 #pragma unroll 4
@@ -361,7 +364,7 @@ __global__ void __launch_bounds__(kEmThreads, (DP * KP <= 128 || MODE == 2) ? 4 
             __syncthreads();
         }
 
-        if (MODE != 2) {
+        if (MODE < 2) {
             double* out = p.partials + static_cast<long long>(chunk) * SV;
 #pragma unroll
             for (int i = 0; i < MW; ++i) {
@@ -700,7 +703,7 @@ struct mlb_em {
     int64_t direct_steps = 0;    // steps that took the direct kernels so far (mlb_em_direct_steps)
     int64_t launches = 0;
     int64_t steps_done = 0;
-    EmKernelFn fn_step = nullptr, fn_mstep = nullptr, fn_emit = nullptr;
+    EmKernelFn fn_step = nullptr, fn_mstep = nullptr, fn_emit = nullptr, fn_score = nullptr;
     int path = 1;                // feature-space kernels of this shape: 1 fused E+M (D <= 16, K <= 32), 2 split E / M; 0: none (D > 64 or K > 256)
     EmDirect dr;                 // direct-difference kernels
     int forced_path = 0;         // mlb_em_force_path: 0 automatic, 3 always direct
@@ -708,7 +711,7 @@ struct mlb_em {
     double kappa_max = 0.0;      // max_k (mu_k - c)^T P_k (mu_k - c) of the current parameters
     bool r_direct_valid = false; // the direct R buffer holds the responsibilities of the last step
     double* kappa_host = nullptr;   // pinned: kappa of the current parameters on its way to the routing decision
-    EmSplitKernelFn fn_split_e = nullptr, fn_split_m = nullptr;
+    EmSplitKernelFn fn_split_e = nullptr, fn_split_m = nullptr, fn_split_score = nullptr;
     size_t smem_split_e = 0, smem_split_m = 0;
     size_t smem_fused = 0;       // dynamic shared memory of the fused kernels (em_small_kernel for D <= 8, em_kernel for D = 16)
     int MW = 4;                  // split M kernel: feature tiles per warp
@@ -883,6 +886,10 @@ static EmDirectKernelFn direct_e_kernel_for(int NB)
 {
     return NB == 1 ? em_direct_e_kernel<1> : NB == 2 ? em_direct_e_kernel<2> : em_direct_e_kernel<0>;
 }
+static EmDirectKernelFn direct_score_kernel_for(int NB)
+{
+    return NB == 1 ? em_direct_e_kernel<1 + kDrScore> : NB == 2 ? em_direct_e_kernel<2 + kDrScore> : em_direct_e_kernel<kDrScore>;
+}
 
 // Super-chunks: every virtual shard's chunks are cut into at most kDrSuperPerVshard contiguous runs (a function of N only).
 static void direct_layout(mlb_em* em, int vshard, std::vector<int64_t>& point_bounds)
@@ -930,6 +937,7 @@ static int direct_prepare(mlb_em* em)
         MLB_CUDA(cudaMemcpyAsync(dg.tile_tab, tiles.data(), sizeof(int2) * tiles.size(), cudaMemcpyHostToDevice, gpu.stream));
         const auto e_kernel = direct_e_kernel_for(dr.NB);
         MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(e_kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(dr.smem_e)));
+        MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(direct_score_kernel_for(dr.NB)), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(dr.smem_e)));
         MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(em_direct_m_kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(dr.smem_m)));
         int per_e = 0, per_m = 0, sms = 0;
         MLB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_e, reinterpret_cast<const void*>(e_kernel), kDrThreads, dr.smem_e));
@@ -1278,6 +1286,81 @@ __global__ void em_onehot_kernel(const unsigned* __restrict__ labels, long long 
     for (int kk = 0; kk < k; ++kk) r[i + static_cast<long long>(kk) * n] = label == static_cast<unsigned>(kk) ? 1.0 : 0.0;
 }
 
+// ---------------------------------------------------------------- scoring: log p(x) under the current parameters
+//
+// The scoring kernels (em_kernel / em_small_kernel MODE 3, em_split_e_kernel and em_direct_e_kernel with the score flag) write one value
+// per point and touch nothing a step reads or writes: not the theta slots, the log-likelihood ring, the chunk partials,
+// the resident responsibilities or the kernel timer.  The sums over points are taken from those values by one kernel for
+// every path, so the order in which a mean is summed does not depend on which kernel produced the values.
+constexpr int kScoreSumChunk = 2048;   // points per partial sum of mlb_em_score (kStagePoints is a multiple)
+
+// The sum of every `chunk`-point run of ll[0, n) into out[run]: lane-strided, then a butterfly.  One warp per run.
+__global__ void em_score_sum_kernel(const double* __restrict__ ll, long long n, int chunk, double* __restrict__ out)
+{
+    const long long p0 = static_cast<long long>(blockIdx.x) * chunk, p1 = min64(p0 + chunk, n);
+    double acc = 0.0;
+    for (long long i = p0 + threadIdx.x; i < p1; i += 32) acc += ll[i];
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+    if (threadIdx.x == 0) out[blockIdx.x] = acc;
+}
+
+static int launch_score_sums(mlb_em* em, int g, const double* ll, int64_t n, int chunk, double* out)
+{
+    if (n == 0) return MLB_OK;
+    em_score_sum_kernel<<<static_cast<unsigned>((n + chunk - 1) / chunk), 32, 0, em->ctx->gpus[g].stream>>>(ll, n, chunk, out);
+    MLB_CUDA(cudaGetLastError());
+    ++em->launches;
+    return MLB_OK;
+}
+
+// log p(x) of the n points at x (device memory of GPU g, d doubles each) into ll_out[0, n), on the kernels predict takes
+// with the current parameters.  r_tmp: n * KPr doubles of scratch for the direct kernels' log-densities (route 3 only).
+static int launch_score(mlb_em* em, int g, const double* x, int64_t n, double* ll_out, double* r_tmp)
+{
+    if (n == 0) return MLB_OK;
+    Gpu& gpu = em->ctx->gpus[g];
+    EmGpu& eg = em->gpus[g];
+    if (em->route == 3) {
+        EmDirectArgs a = direct_args(em, g);
+        a.x = x;
+        a.n_local = n;
+        a.r = r_tmp;
+        a.ll_tile = ll_out;
+        const long long ntiles = (n + kDrTile - 1) / kDrTile;
+        MLB_CUDA(cudaMemsetAsync(a.counter, 0, sizeof(unsigned), gpu.stream));
+        direct_score_kernel_for(em->dr.NB)<<<static_cast<unsigned>(std::min<long long>(em->dr.gpus[g].grid_e, ntiles)), kDrThreads, em->dr.smem_e, gpu.stream>>>(a);
+        MLB_CUDA(cudaGetLastError());
+        ++em->launches;
+    } else if (em->path == 2) {
+        EmSplitArgs a = split_args(em, g, eg.theta[em->cur]);
+        a.x = x;
+        a.n_local = n;
+        a.chunk = 128;
+        a.n_chunks = static_cast<int>((n + 127) / 128);
+        a.r = nullptr;
+        a.ll_tile = nullptr;
+        a.r_out = ll_out;
+        MLB_CUDA(cudaMemsetAsync(a.counter, 0, sizeof(unsigned), gpu.stream));
+        const long long e_items = static_cast<long long>(a.n_chunks) * (a.chunk / kSpTile);
+        em->fn_split_score<<<static_cast<unsigned>(std::min<long long>(eg.grid_e, e_items)), kSpThreads, em->smem_split_e, gpu.stream>>>(a);
+        MLB_CUDA(cudaGetLastError());
+        ++em->launches;
+    } else {
+        EmArgs a = base_args(em, g);
+        a.x = x;
+        a.n_local = n;
+        a.theta = eg.theta[em->cur];
+        a.chunk = kTile;
+        a.n_chunks = static_cast<int>((n + kTile - 1) / kTile);
+        a.range_begin = 0;
+        a.range_count = n;
+        a.r_out = ll_out;
+        MLB_TRY(launch_em(em, em->fn_score, a, g, 8 * kSmCount));
+    }
+    return MLB_OK;
+}
+
 }  // namespace mlb
 
 extern "C" {
@@ -1332,9 +1415,11 @@ int mlb_em_create(mlb_ctx* ctx, mlb_data* data, int k, mlb_em** out)
         em->fn_step = em_kernel_for<0>(DP, KP);
         em->fn_mstep = em_kernel_for<1>(DP, KP);
         em->fn_emit = em_kernel_for<2>(DP, KP);
+        em->fn_score = em_kernel_for<3>(DP, KP);
         em->smem_fused = DP <= 8 ? em_small_smem_bytes(DP, KP) : em_smem_bytes(DP, KP);
     } else if (split) {
         em->fn_split_e = NT == 8 ? em_split_e_kernel<8> : NT == 4 ? em_split_e_kernel<4> : em_split_e_kernel<2>;
+        em->fn_split_score = NT == 8 ? em_split_e_kernel<8 + kSpScore> : NT == 4 ? em_split_e_kernel<4 + kSpScore> : em_split_e_kernel<2 + kSpScore>;
         // feature tiles per warp of the M kernel: the choice that wastes the fewest tile slots (ties: the larger)
         int best_waste = 1 << 30;
         for (int mw = 3; mw <= 5; ++mw) {
@@ -1449,7 +1534,7 @@ int mlb_em_create(mlb_ctx* ctx, mlb_data* data, int k, mlb_em** out)
         }
         if (em->path == 1) {
             const size_t smem = em->smem_fused;
-            for (EmKernelFn fn : {em->fn_step, em->fn_mstep, em->fn_emit})
+            for (EmKernelFn fn : {em->fn_step, em->fn_mstep, em->fn_emit, em->fn_score})
                 MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
             int per_sm = 0;
             MLB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reinterpret_cast<const void*>(em->fn_step), em->DP <= 8 ? kSmallThreads : kEmThreads, smem));
@@ -1469,6 +1554,7 @@ int mlb_em_create(mlb_ctx* ctx, mlb_data* data, int k, mlb_em** out)
             }
             MLB_CUDA(cudaMemsetAsync(eg.partials, 0, sizeof(double) * std::max<int64_t>(1, sh.n_chunks()) * em->SV, gpu.stream));
             MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(em->fn_split_e), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(em->smem_split_e)));
+            MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(em->fn_split_score), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(em->smem_split_e)));
             MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(em->fn_split_m), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(em->smem_split_m)));
             int per_e = 0, per_m = 0;
             MLB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_e, reinterpret_cast<const void*>(em->fn_split_e), kSpThreads, em->smem_split_e));
@@ -1912,6 +1998,118 @@ int mlb_em_predict(mlb_em* em, const double* x, int64_t m, int64_t ld_x, double*
     rc = body();
     for (double* ptr : {xd, r_tmp, ll_tmp})
         if (ptr) cudaFreeAsync(ptr, gpu.stream);
+    return rc;
+}
+
+int mlb_em_score(mlb_em* em, const double* x, int64_t m, int64_t ld_x, double* log_density_out, double* mean_out)
+{
+    MLB_ENTER(em ? em->ctx : nullptr);
+    MLB_REQUIRE(em && x, "mlb_em_score: null argument");
+    MLB_REQUIRE(m >= 0 && ld_x >= em->d, "mlb_em_score: bad shape (m=%lld, ld_x=%lld, D=%d)", static_cast<long long>(m), static_cast<long long>(ld_x), em->d);
+    if (!em->have_params) { set_error("mlb_em_score: parameters not set"); return MLB_ESTATE; }
+    if (mean_out) *mean_out = std::numeric_limits<double>::quiet_NaN();   // the mean of no points
+    if (m == 0 || (!log_density_out && !mean_out)) return MLB_OK;
+    Gpu& gpu = em->ctx->gpus[0];
+    const int d = em->d;
+    const bool direct = em->route == 3;
+    if (direct) MLB_TRY(direct_prepare(em));
+    MLB_CUDA(cudaSetDevice(gpu.device));
+    const int64_t cap = std::min<int64_t>(m, kStagePoints);
+    double *xd = nullptr, *ll = nullptr, *sums = nullptr, *r_tmp = nullptr;
+    std::vector<double> host_sums;
+    auto body = [&]() -> int {
+        MLB_CUDA(cudaMallocFromPoolAsync(&xd, sizeof(double) * cap * d, gpu.pool, gpu.stream));
+        MLB_CUDA(cudaMallocFromPoolAsync(&ll, sizeof(double) * cap, gpu.pool, gpu.stream));
+        MLB_CUDA(cudaMallocFromPoolAsync(&sums, sizeof(double) * ((cap + kScoreSumChunk - 1) / kScoreSumChunk), gpu.pool, gpu.stream));
+        if (direct) MLB_CUDA(cudaMallocFromPoolAsync(&r_tmp, sizeof(double) * cap * em->dr.KPr, gpu.pool, gpu.stream));
+        for (int64_t off = 0; off < m; off += kStagePoints) {
+            const int64_t n = std::min<int64_t>(kStagePoints, m - off);
+            MLB_TRY(staged_h2d(gpu, xd, x + off * ld_x, static_cast<size_t>(n), sizeof(double) * d, sizeof(double) * ld_x));
+            MLB_TRY(launch_score(em, 0, xd, n, ll, r_tmp));
+            if (mean_out) {
+                // partial sums over runs of kScoreSumChunk points: the stages are whole runs, so the sums do not depend on them
+                const size_t nsums = static_cast<size_t>((n + kScoreSumChunk - 1) / kScoreSumChunk), first = host_sums.size();
+                MLB_TRY(launch_score_sums(em, 0, ll, n, kScoreSumChunk, sums));
+                host_sums.resize(first + nsums);
+                MLB_CUDA(cudaMemcpyAsync(host_sums.data() + first, sums, sizeof(double) * nsums, cudaMemcpyDeviceToHost, gpu.stream));
+            }
+            if (log_density_out) MLB_TRY(staged_d2h(gpu, log_density_out + off, ll, sizeof(double) * n));
+            MLB_CUDA(cudaStreamSynchronize(gpu.stream));
+        }
+        return MLB_OK;
+    };
+    int rc = body();
+    for (double* ptr : {xd, ll, sums, r_tmp})
+        if (ptr) cudaFreeAsync(ptr, gpu.stream);
+    const cudaError_t sync = cudaStreamSynchronize(gpu.stream);
+    if (rc == MLB_OK && sync != cudaSuccess) { set_error("mlb_em_score: %s", cudaGetErrorString(sync)); rc = MLB_ECUDA; }
+    if (rc == MLB_OK && mean_out) {
+        double total = 0.0;
+        for (double v : host_sums) total += v;   // in point order
+        *mean_out = total / static_cast<double>(m);
+    }
+    return rc;
+}
+
+int mlb_em_score_fitted(mlb_em* em, double* log_density_out, double* mean_out)
+{
+    MLB_ENTER(em ? em->ctx : nullptr);
+    MLB_REQUIRE(em, "mlb_em_score_fitted: null argument");
+    if (!em->have_params) { set_error("mlb_em_score_fitted: parameters not set"); return MLB_ESTATE; }
+    mlb_ctx* ctx = em->ctx;
+    const Layout& lay = em->data->lay;
+    const int d = em->d;
+    const bool direct = em->route == 3;
+    if (direct) MLB_TRY(direct_prepare(em));
+    // Stages of whole chunks (every shard starts on a chunk boundary), so each chunk's sum is taken over the same points
+    // in the same order whatever the stage size; the chunk sums then take the reduction and exchange of a step.
+    const int64_t stage = std::max<int64_t>(lay.chunk, kStagePoints / lay.chunk * lay.chunk);
+    const int64_t host_begin = ctx->rank_mode ? em->data->shards[0].begin : 0;
+    const size_t ng = ctx->gpus.size();
+    std::vector<double*> ll(ng, nullptr), part(ng, nullptr), vsum(ng, nullptr), r_tmp(ng, nullptr);
+    ReduceScratch scratch;
+    double host_vsum[kVirtualShards] = {};
+    auto body = [&]() -> int {
+        MLB_TRY(for_each_gpu(ctx, [&](int g, Gpu& gpu) -> int {
+            const DataShard& sh = em->data->shards[g];
+            const int64_t cap = std::max<int64_t>(1, std::min(stage, sh.n()));
+            MLB_CUDA(cudaMallocFromPoolAsync(&ll[g], sizeof(double) * cap, gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMallocFromPoolAsync(&part[g], sizeof(double) * std::max<int64_t>(1, sh.n_chunks()), gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMallocFromPoolAsync(&vsum[g], sizeof(double) * kVirtualShards, gpu.pool, gpu.stream));
+            if (direct) MLB_CUDA(cudaMallocFromPoolAsync(&r_tmp[g], sizeof(double) * cap * em->dr.KPr, gpu.pool, gpu.stream));
+            return MLB_OK;
+        }));
+        for (int64_t off = 0;; off += stage) {
+            bool any = false;
+            MLB_TRY(for_each_gpu(ctx, [&](int g, Gpu& gpu) -> int {
+                const DataShard& sh = em->data->shards[g];
+                const int64_t n = std::min(stage, sh.n() - off);
+                if (n <= 0) return MLB_OK;
+                any = true;
+                MLB_TRY(launch_score(em, g, sh.x + off * d, n, ll[g], r_tmp[g]));
+                MLB_TRY(launch_score_sums(em, g, ll[g], n, lay.chunk, part[g] + off / lay.chunk));
+                if (log_density_out) MLB_TRY(staged_d2h(gpu, log_density_out + (sh.begin - host_begin) + off, ll[g], sizeof(double) * n));
+                return MLB_OK;
+            }));
+            if (!any) break;
+        }
+        MLB_TRY(reduce_and_exchange(em->data, part, vsum, 1, scratch));
+        em->launches += static_cast<int64_t>(ng);
+        Gpu& gpu0 = ctx->gpus[0];
+        MLB_CUDA(cudaSetDevice(gpu0.device));
+        MLB_CUDA(cudaMemcpyAsync(host_vsum, vsum[0], sizeof(host_vsum), cudaMemcpyDeviceToHost, gpu0.stream));
+        return MLB_OK;
+    };
+    int rc = body();
+    const int rc_sync = mlb_ctx_synchronize(ctx);
+    if (rc == MLB_OK) rc = rc_sync;
+    for (size_t g = 0; g < ng; ++g) {
+        cudaSetDevice(ctx->gpus[g].device);
+        for (double* ptr : {ll[g], part[g], vsum[g], r_tmp[g]})
+            if (ptr) cudaFreeAsync(ptr, ctx->gpus[g].stream);
+    }
+    scratch.release(ctx);
+    if (rc == MLB_OK && mean_out) *mean_out = tree8(host_vsum, 1) / static_cast<double>(lay.n_total);
     return rc;
 }
 

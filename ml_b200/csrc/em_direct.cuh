@@ -51,7 +51,7 @@ struct EmDirectArgs {
     const double* shift;    // d
     const double* img;      // [k][dr_img_len(DP)] component images (em_finalize_kernel)
     double* r;              // [n_local][KPr]
-    double* ll_tile;        // [ceil(n_local / 64)] log-likelihood sum of every E tile
+    double* ll_tile;        // [ceil(n_local / 64)] log-likelihood sum of every E tile; scoring: [n_local] log p(x) of every point
     unsigned* counter;
     int cb;                 // E: components per staged batch
     // M
@@ -77,9 +77,15 @@ inline size_t em_direct_m_smem(int DP, int cg, int d)
 
 // ---------------------------------------------------------------- E kernel (expectation_step, EM.cpp:190-219)
 // NBT: the number of 8-coordinate blocks when it is 1 or 2 (D <= 16: the loops over the blocks unroll completely), 0 for any D.
-template <int NBT>
+// NBTS = NBT, or NBT + kDrScore for the scoring pass, which writes log p(x) per point to ll_tile instead of responsibilities
+// and tile sums (r receives the log-densities only).  The flag rides in the one int parameter so that the step's instances
+// keep their names and their code.
+constexpr int kDrScore = 16;
+template <int NBTS>
 __global__ void __launch_bounds__(kDrThreads) em_direct_e_kernel(const EmDirectArgs p)
 {
+    constexpr int NBT = NBTS & (kDrScore - 1);
+    constexpr bool SCORE = (NBTS & kDrScore) != 0;
     extern __shared__ __align__(16) double sm[];
     const int DP = NBT ? 8 * NBT : p.DP, NB = DP / 8, ZS = DP + 4, IMG = dr_img_len(DP), SPC = dr_steps(NB), d = p.d;
     double* Z = sm;                                     // [64][ZS]
@@ -201,7 +207,9 @@ __global__ void __launch_bounds__(kDrThreads) em_direct_e_kernel(const EmDirectA
                 for (int kk = hl; kk < p.k; kk += 16) sum += exp_nonpositive(__ldcg(rrow + kk) - mx, etab);
 #pragma unroll
             for (int off = 8; off >= 1; off >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, off);
-            if (live) {
+            if constexpr (SCORE) {
+                if (live && hl == 0) p.ll_tile[tile0 + pl] = (mx + log(sum)) - 0.5 * d * kLog2Pi;
+            } else if (live) {
                 const double inv = reciprocal_of_sum(sum);
                 for (int kk = hl; kk < p.KPr; kk += 16) rrow[kk] = exp_nonpositive(__ldcg(rrow + kk) - mx, etab) * inv;   // padding: exp(-inf) = 0
                 if (hl == 0) {
@@ -209,6 +217,10 @@ __global__ void __launch_bounds__(kDrThreads) em_direct_e_kernel(const EmDirectA
                     ll_prod *= sum;
                 }
             }
+        }
+        if constexpr (SCORE) {
+            __syncthreads();   // Z is rewritten by the next item
+            continue;
         }
         ll_acc += log(ll_prod);
 #pragma unroll

@@ -33,7 +33,7 @@ constexpr size_t em_small_smem_bytes(int DP, int KP)
 }
 
 template <int DP, int KP, int MODE>
-__global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(DP) * (KP / 8) <= 6) ? 5 : (em_small_nm(DP) * (KP / 8) <= 12) ? 4 : 3)) em_small_kernel(const EmArgs p)
+__global__ void __launch_bounds__(kSmallThreads, MODE >= 2 ? 4 : ((em_small_nm(DP) * (KP / 8) <= 6) ? 5 : (em_small_nm(DP) * (KP / 8) <= 12) ? 4 : 3)) em_small_kernel(const EmArgs p)
 {
     constexpr int NT = KP / 8, DQ = DP / 4, NE = em_ne(DP), NM = em_small_nm(DP);
     constexpr int RS = KP + 4, PS = NM * 8 + 4;
@@ -66,8 +66,8 @@ __global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(D
     double* F = Phi + warp * kSmallSub * PS;
     double* R = Rw + warp * kSmallSub * RS;
 
-    const long long work_begin = MODE == 2 ? p.range_begin : 0;
-    const long long work_end = MODE == 2 ? p.range_begin + p.range_count : p.n_local;
+    const long long work_begin = MODE >= 2 ? p.range_begin : 0;
+    const long long work_end = MODE >= 2 ? p.range_begin + p.range_count : p.n_local;
 
     double xr[XR];
     auto load_sub = [&](long long point0, int nvalid) {
@@ -104,7 +104,7 @@ __global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(D
         const int nsubs = static_cast<int>((p_end - p_begin + kSmallSub - 1) / kSmallSub);
 
         double sacc[NM][NT][2];
-        if (MODE != 2) {
+        if (MODE < 2) {
 #pragma unroll
             for (int i = 0; i < NM; ++i)
 #pragma unroll
@@ -144,7 +144,7 @@ __global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(D
             }
             // One E-step slot group: the products go to the feature table and (unless the responsibilities are given) into Q.
             auto estep = [&](int j, double a0, double a1, bool keep) {
-                if (MODE != 2 && keep) {
+                if (MODE < 2 && keep) {
                     f0[4 * j] = a0;
                     f1[4 * j] = a1;
                 }
@@ -228,6 +228,8 @@ __global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(D
 #pragma unroll
                         for (int nt = 0; nt < NT; ++nt)
                             *reinterpret_cast<double2*>(R + pl * RS + 8 * nt + 2 * c) = make_double2(acc[mt][nt][0] * inv, acc[mt][nt][1] * inv);
+                    } else if (MODE == 3) {
+                        if (c == 0 && pl < nvalid) p.r_out[(tile0 - p.range_begin) + pl] = (mxs[mt] + log(sums[mt])) - 0.5 * d * kLog2Pi;
                     } else {
                         // emit: responsibilities_ (EM.cpp:213-218) and labels_ (EM.cpp:289-304, first maximum wins)
                         double best = -1.0;
@@ -258,7 +260,7 @@ __global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(D
                     nlogged = 0;
                 }
             }
-            if (MODE != 2) {
+            if (MODE < 2) {
                 __syncwarp();
                 // ---------------- M-step: S += Phi^T . R over the warp's 16 points, all rows and components in registers
 #pragma unroll
@@ -278,7 +280,7 @@ __global__ void __launch_bounds__(kSmallThreads, MODE == 2 ? 4 : ((em_small_nm(D
             }
         }
 
-        if (MODE != 2) {
+        if (MODE < 2) {
             ll_acc += log(ll_prod);
             // ---------------- chunk partial: the warps' statistics added in the fixed order ((w0 + w1) + w2) + w3 ...
             double* red = Phi;   // NM * 8 * KP doubles; every warp is past its last read of the feature table

@@ -24,6 +24,7 @@ namespace mlb {
 constexpr int kSpTile = 64;      // points per tile
 constexpr int kSpThreads = 128;  // 4 warps
 constexpr int kSpJB = 8;         // E-step feature steps per staged Theta block
+constexpr double kLog2Pi = 0x1.d67f1c864beb4p+0;   // log(2 pi): log p(x) = log-sum-exp of the E-step terms - D/2 log(2 pi)
 
 struct EmSplitArgs {
     const double* x;        // local points, d doubles each
@@ -41,7 +42,7 @@ struct EmSplitArgs {
     int chunk, n_chunks;
     unsigned* counter;
     // emit
-    double* r_out;          // column-major staging, leading dimension r_out_ld
+    double* r_out;          // column-major staging, leading dimension r_out_ld; scoring: log p(x) of every local point
     long long r_out_ld;
     unsigned* labels_out;
     long long range_begin, range_count;
@@ -94,9 +95,14 @@ inline size_t em_split_e_smem(int NT, int DP, int KP)
 }
 
 // ---------------------------------------------------------------- E kernel
-template <int NT>
+// NTS = NT, or NT + kSpScore for the scoring pass, which writes log p(x) per point to r_out instead of R and the tile sums.
+// (A flag inside the one int parameter keeps the names, and so the code, of the step's instances as they were.)
+constexpr int kSpScore = 256;
+template <int NTS>
 __global__ void __launch_bounds__(kSpThreads, 2) em_split_e_kernel(const EmSplitArgs p)
 {
+    constexpr int NT = NTS & (kSpScore - 1);
+    constexpr bool SCORE = (NTS & kSpScore) != 0;
     constexpr int KG = 8 * NT;
     extern __shared__ __align__(16) double sm[];
     const int DP = p.DP, KP = p.KP, d = p.d, ZS = DP + 4, QS = KP + 4;
@@ -153,7 +159,7 @@ __global__ void __launch_bounds__(kSpThreads, 2) em_split_e_kernel(const EmSplit
         {
             const long long tile0 = p_begin + static_cast<long long>(t) * kSpTile;
             if (tile0 >= p_end) {
-                if (tid == 0) p.ll_tile[item] = 0.0;
+                if (!SCORE && tid == 0) p.ll_tile[item] = 0.0;
                 continue;
             }
             const int nvalid = static_cast<int>(p_end - tile0 < kSpTile ? p_end - tile0 : kSpTile);
@@ -216,11 +222,15 @@ __global__ void __launch_bounds__(kSpThreads, 2) em_split_e_kernel(const EmSplit
                 double sum = 0.0;
                 for (int kk = hl; kk < KP; kk += 16) {
                     const double e = exp_nonpositive(qrow[kk] - mx, etab);
-                    qrow[kk] = e;
+                    if (!SCORE) qrow[kk] = e;
                     sum += e;
                 }
 #pragma unroll
                 for (int off = 8; off >= 1; off >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, off);
+                if constexpr (SCORE) {
+                    if (pl < nvalid && hl == 0) p.r_out[tile0 + pl] = (mx + log(sum)) - 0.5 * d * kLog2Pi;
+                    continue;
+                }
                 const double inv = reciprocal_of_sum(sum);
                 if (pl < nvalid) {
                     double* rrow = p.r + (tile0 + pl) * KP;
@@ -232,6 +242,10 @@ __global__ void __launch_bounds__(kSpThreads, 2) em_split_e_kernel(const EmSplit
                 }
             }
             ll_acc += log(ll_prod);
+        }
+        if constexpr (SCORE) {
+            __syncthreads();   // Z and Q are rewritten by the next item
+            continue;
         }
 
         // log-likelihood sum of the tile: fixed butterfly inside the warp, fixed order across warps

@@ -9,6 +9,8 @@
 //   - number_iterations(): iterations run by the last fit (requested by the north star; the
 //     reference does not store it);
 //   - assign_responsibilities(points): the batched form of assign_responsibilities(x, u), on the device;
+//   - log_likelihoods(points), log_likelihood(points), log_likelihoods() and final_log_likelihood(): log p(x) under the
+//     returned parameters, per point and as a mean, for new points or the fitted ones, on the device;
 //   - the built-in KPP and ClosestCentroid initialisers run their O(N K D) distance passes on the device (the draws
 //     stay on the host with the model's PRNG, so the initial state is the reference's);
 //   - responsibilities() and labels() are out of line: the N x K matrix (25.6 GB at N=1e8, K=32) and the N labels
@@ -85,7 +87,28 @@ namespace ml
 		/** N x K, from the last E-step of the fit. */
 		DLL_DECLSPEC const Eigen::MatrixXd& responsibilities() const;
 
+		/** Mean log-likelihood per point at the parameters of the last E-step of the fit (before its M-step). */
 		double log_likelihood() const { return log_likelihood_; }
+
+		/** log p(x) = log sum_k w_k N(x | mu_k, Sigma_k) of every column of `points` (D x m) under the current parameters,
+		on the device.
+		@throw std::invalid_argument If `points` has the wrong number of rows.
+		@throw std::logic_error If there is no fitted device state (no fit yet, the N == K exact fit, or after release_device()). */
+		DLL_DECLSPEC Eigen::VectorXd log_likelihoods(DataView points) const;
+
+		/** The mean of log_likelihoods(points).
+		@throw std::invalid_argument If `points` has the wrong number of rows.
+		@throw std::logic_error If there is no fitted device state. */
+		DLL_DECLSPEC double log_likelihood(DataView points) const;
+
+		/** log p(x) of every fitted point (this process's own points under ml::Distributed) under the current parameters.
+		@throw std::logic_error If there is no fitted device state. */
+		DLL_DECLSPEC Eigen::VectorXd log_likelihoods() const;
+
+		/** The mean log-likelihood of the fitted points at the parameters the fit returned (log_likelihood() belongs to the
+		parameters before the last M-step).  Under ml::Distributed: over all ranks' points, and collective.
+		@throw std::logic_error If there is no fitted device state. */
+		DLL_DECLSPEC double final_log_likelihood() const;
 
 		std::shared_ptr<const Clustering::CentroidsInitialiser> means_initialiser() const { return means_initialiser_; }
 

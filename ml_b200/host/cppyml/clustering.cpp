@@ -10,6 +10,7 @@
 #include <pybind11/numpy.h>
 #include <pybind11/stl.h>
 
+#include <cmath>
 #include <cstring>
 #include <stdexcept>
 
@@ -91,6 +92,7 @@ namespace ml
 		bool fit_row_major(const py::array& data)
 		{
 			const auto columns = as_columns(data);
+			fitted_points_ = columns.cols();
 			py::gil_scoped_release release;   // no Python callbacks happen inside fit
 			return fit(columns);
 		}
@@ -114,6 +116,46 @@ namespace ml
 			}
 			return to_numpy(result);
 		}
+
+		/** log p(x) of every row of `data` (m, D), or of the fitted points when `data` is None, on the device. */
+		py::array_t<double> score_samples_py(const py::object& data) const
+		{
+			Eigen::VectorXd result;
+			if (data.is_none()) {
+				py::gil_scoped_release release;
+				result = log_likelihoods();
+			} else {
+				const auto columns = as_columns(data);
+				py::gil_scoped_release release;
+				result = log_likelihoods(columns);
+			}
+			return to_numpy(result);
+		}
+
+		/** Mean log p(x) over the rows of `data`, or over the fitted points when `data` is None. */
+		double score_py(const py::object& data) const
+		{
+			if (data.is_none()) {
+				py::gil_scoped_release release;
+				return final_log_likelihood();
+			}
+			const auto columns = as_columns(data);
+			py::gil_scoped_release release;
+			return log_likelihood(columns);
+		}
+
+		/** -2 n score(data) + penalty_per_parameter * p, p the free parameters of a full-covariance mixture (sklearn's
+		GaussianMixture._n_parameters: K D means, K D (D + 1) / 2 covariance entries, K - 1 weights). */
+		double information_criterion(const py::object& data, bool bayesian) const
+		{
+			const double n = static_cast<double>(data.is_none() ? fitted_points_ : as_columns(data).cols());
+			const double d = static_cast<double>(means().rows()), k = static_cast<double>(number_components());
+			const double p = k * d + k * d * (d + 1) / 2 + k - 1;
+			return -2 * n * score_py(data) + (bayesian ? std::log(n) : 2.0) * p;
+		}
+
+	private:
+		Eigen::Index fitted_points_ = 0;
 	};
 
 	namespace Clustering
@@ -225,7 +267,7 @@ void init_clustering(py::module_& m)
 			py::detail::array_proxy(view.ptr())->flags &= ~py::detail::npy_api::NPY_ARRAY_WRITEABLE_;
 			return view;
 		}, "Responsibilities of the last E-step, shape (N, K): a read-only view of the model's matrix, brought to the host on first access.")
-		.def_property_readonly("log_likelihood", &ml::EMPy::log_likelihood, "Mean log-likelihood per point at the last E-step.")
+		.def_property_readonly("log_likelihood", [](const ml::EMPy& em) { return em.log_likelihood(); }, "Mean log-likelihood per point at the last E-step.")
 		.def_property_readonly("mixing_probabilities", [](const ml::EMPy& em) { return to_numpy(em.mixing_probabilities()); }, "Mixture weights, shape (K,).")
 		.def_property_readonly("number_iterations", &ml::EMPy::number_iterations, "Iterations run by the last fit.")
 		.def_property_readonly("converged", &ml::EMPy::converged, "Whether the last fit converged.")
@@ -237,6 +279,14 @@ void init_clustering(py::module_& m)
 		.def("release_device", &ml::EMPy::release_device, py::arg("keep_results") = true, "Frees the GPU memory the last fit still holds (the points and the pending results); with keep_results the responsibilities and labels are brought to the host first.")
 		.def("assign_responsibilities_batch", &ml::EMPy::calculate_responsibilities_batch, py::arg("data").noconvert(),
 			"Responsibilities of the fitted components for every row of data (computed on the GPU).\n\nArgs:\n    data: A 2D float64 C-contiguous array with data points in rows.\n\nReturns:\n    2D array, one row of responsibilities per data point.")
+		.def("score_samples", &ml::EMPy::score_samples_py, py::arg("data").noconvert() = py::none(),
+			"Log-likelihood log p(x) of every point under the fitted mixture (computed on the GPU), as sklearn's GaussianMixture.score_samples.\n\nArgs:\n    data: A 2D float64 C-contiguous array of shape (m, D) with points in rows, or None for the fitted points (still on the GPU).\n\nReturns:\n    Array of shape (m,).")
+		.def("score", &ml::EMPy::score_py, py::arg("data").noconvert() = py::none(),
+			"Mean log-likelihood per point under the fitted mixture, as sklearn's GaussianMixture.score.  With data=None it is the log-likelihood of the parameters the fit returned (the log_likelihood property belongs to the parameters before the last M-step).\n\nArgs:\n    data: A 2D float64 C-contiguous array of shape (m, D), or None for the fitted points.")
+		.def("bic", [](const ml::EMPy& em, const py::object& data) { return em.information_criterion(data, true); }, py::arg("data").noconvert() = py::none(),
+			"Bayesian information criterion -2 n score(data) + p ln n, p = K D + K D (D + 1) / 2 + K - 1 free parameters (sklearn's definition).\n\nArgs:\n    data: A 2D float64 C-contiguous array of shape (n, D), or None for the fitted points.")
+		.def("aic", [](const ml::EMPy& em, const py::object& data) { return em.information_criterion(data, false); }, py::arg("data").noconvert() = py::none(),
+			"Akaike information criterion -2 n score(data) + 2 p (sklearn's definition).\n\nArgs:\n    data: A 2D float64 C-contiguous array of shape (n, D), or None for the fitted points.")
 		.doc() = "Full-covariance Gaussian mixture fitted by expectation-maximisation on B200 GPUs.";
 
 	py::class_<ml::Clustering::KMeansPy, std::shared_ptr<ml::Clustering::KMeansPy>>(m_clustering, "KMeans")

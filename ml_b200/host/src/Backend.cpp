@@ -179,6 +179,22 @@ namespace ml
 			check(mlb_em_predict(em_, points.data(), points.cols(), points.outerStride(), responsibilities.data(), std::max<Eigen::Index>(1, points.cols()), nullptr), "EM responsibilities of new points");
 		}
 
+		void EmDevice::score(Eigen::Ref<const Eigen::MatrixXd> points, Eigen::VectorXd* log_densities, double* mean)
+		{
+			if (log_densities) {
+				log_densities->resize(points.cols());
+			}
+			check(mlb_em_score(em_, points.data(), points.cols(), points.outerStride(), log_densities ? log_densities->data() : nullptr, mean), "EM log-likelihood of new points");
+		}
+
+		void EmDevice::score_fitted(Eigen::VectorXd* log_densities, double* mean)
+		{
+			if (log_densities) {
+				log_densities->resize(data_->cols());
+			}
+			check(mlb_em_score_fitted(em_, log_densities ? log_densities->data() : nullptr, mean), "EM log-likelihood of the fitted points");
+		}
+
 		double EmDevice::step()
 		{
 			double log_likelihood = 0;

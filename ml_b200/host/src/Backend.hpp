@@ -73,6 +73,11 @@ namespace ml
 			void maximise_from_labels(const std::vector<unsigned int>& labels);
 			/** Responsibilities (m x K) of the columns of `points` (D x m) under the current parameters. */
 			void predict(Eigen::Ref<const Eigen::MatrixXd> points, Eigen::MatrixXd& responsibilities);
+			/** log p(x) of the columns of `points` (D x m) under the current parameters; either output may be null. */
+			void score(Eigen::Ref<const Eigen::MatrixXd> points, Eigen::VectorXd* log_densities, double* mean);
+			/** The same for the fitted points: this process's own points, and the mean over all points (collective under
+			ml::Distributed). */
+			void score_fitted(Eigen::VectorXd* log_densities, double* mean);
 			const std::shared_ptr<DeviceData>& data() const { return data_; }
 			double step();
 			void get_parameters(Eigen::MatrixXd& means, std::vector<Eigen::MatrixXd>& covariances, Eigen::VectorXd& mixing_probabilities);

@@ -325,6 +325,52 @@ namespace ml
 		return result;
 	}
 
+	Eigen::VectorXd EM::log_likelihoods(DataView points) const
+	{
+		if (points.rows() != means().rows()) {
+			throw std::invalid_argument("Wrong number of rows");
+		}
+		if (!device_) {
+			throw std::logic_error("EM: no fitted device state");
+		}
+		Eigen::VectorXd result;
+		device_->score(points, &result, nullptr);
+		return result;
+	}
+
+	double EM::log_likelihood(DataView points) const
+	{
+		if (points.rows() != means().rows()) {
+			throw std::invalid_argument("Wrong number of rows");
+		}
+		if (!device_) {
+			throw std::logic_error("EM: no fitted device state");
+		}
+		double mean = 0;
+		device_->score(points, nullptr, &mean);
+		return mean;
+	}
+
+	Eigen::VectorXd EM::log_likelihoods() const
+	{
+		if (!device_) {
+			throw std::logic_error("EM: no fitted device state");
+		}
+		Eigen::VectorXd result;
+		device_->score_fitted(&result, nullptr);
+		return result;
+	}
+
+	double EM::final_log_likelihood() const
+	{
+		if (!device_) {
+			throw std::logic_error("EM: no fitted device state");
+		}
+		double mean = 0;
+		device_->score_fitted(nullptr, &mean);
+		return mean;
+	}
+
 	void EM::assign_responsibilities(PointView x, VectorOut u) const
 	{
 		if (x.size() != means().rows()) {
