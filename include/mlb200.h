@@ -278,6 +278,33 @@ int mlb_km_update(mlb_km* km, double* centroid_shift_sq);
  * Does not touch the labels, statistics or centroids of the fit.  Runs on the first local GPU. */
 int mlb_km_predict(mlb_km* km, const double* x, int64_t m, int64_t ld_x, unsigned int* labels_out, double* sqdist_out);
 
+/* Distances and inertia under the CURRENT centroids (after a fit: the ones it returned).  None of these calls changes
+ * what a step, predict or get_labels reads: labels and the previous labels n_changed compares against, the statistics
+ * mlb_km_update applies, centroids, old centroids and kernel timing stay as they were (the launch count grows).
+ *
+ * The distance of each of m host points (column-major D x m, stride ld_x >= D) to every centroid, on the first local GPU:
+ * dist_out is m x K column-major with leading dimension ld_out >= m.  squared = 0 gives Euclidean distances, squared != 0
+ * their squares.  A squared distance is (x - c).squaredNorm() as mlb_km_predict evaluates it (the sequential
+ * fused-multiply-add chain), so dist_out[i + label_i ld_out] is bitwise predict's sqdist_out[i] and the first minimum of a
+ * row is predict's label; the Euclidean distance is sqrt of that value.  Staged in batches of at most 2^20 points and
+ * 1 GiB of distances. */
+int mlb_km_transform(mlb_km* km, const double* x, int64_t m, int64_t ld_x, int squared, double* dist_out, int64_t ld_out);
+
+/* The same for the resident points in the GLOBAL range [begin, begin + count): dist_out is count x K column-major with
+ * leading dimension ld_out >= count.  The range may span the GPUs of a context; rank contexts can only read their own rows. */
+int mlb_km_transform_range(mlb_km* km, int64_t begin, int64_t count, int squared, double* dist_out, int64_t ld_out);
+
+/* Inertia sum_i min_k |x_i - c_k|^2 of m host points (as mlb_km_transform), and sqdist_out[i] (may be NULL) as
+ * mlb_km_predict gives it.  The sum is taken over runs of 2048 points on the device and the run sums are added on the
+ * host in order: bitwise repeatable, and independent of the staging.  The inertia of m = 0 points is 0. */
+int mlb_km_score(mlb_km* km, const double* x, int64_t m, int64_t ld_x, double* sqdist_out, double* inertia_out);
+
+/* The inertia of the resident points under the current centroids: bitwise the inertia the next mlb_km_assign would
+ * report, for G = 1, 2, 4, 8 and for rank contexts (after a fit that stopped at its step limit, the inertia of the
+ * centroids it returned rather than of the last assignment).  Needs 4 bytes per resident point and 64 per chunk of
+ * device scratch for the duration of the call.  Collective in rank contexts. */
+int mlb_km_score_fitted(mlb_km* km, double* inertia_out);
+
 /* labels_ of the last assignment; rank contexts receive their own range. */
 int mlb_km_get_labels(mlb_km* km, unsigned int* labels);
 int mlb_km_launch_count(const mlb_km* km, int64_t* launches);

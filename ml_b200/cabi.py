@@ -83,6 +83,10 @@ SIGNATURES = {
     "mlb_km_assign": (ctypes.c_int, [_vp, _c_dp, _c_i64p]),
     "mlb_km_update": (ctypes.c_int, [_vp, _c_dp]),
     "mlb_km_predict": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, ctypes.c_int64, _vp, _vp]),
+    "mlb_km_transform": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, _vp, ctypes.c_int64]),
+    "mlb_km_transform_range": (ctypes.c_int, [_vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, _vp, ctypes.c_int64]),
+    "mlb_km_score": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, ctypes.c_int64, _vp, _c_dp]),
+    "mlb_km_score_fitted": (ctypes.c_int, [_vp, _c_dp]),
     "mlb_km_get_labels": (ctypes.c_int, [_vp, _vp]),
     "mlb_km_launch_count": (ctypes.c_int, [_vp, _c_i64p]),
     "mlb_km_kernel_config": (ctypes.c_int, [_vp, _c_ip]),
@@ -516,6 +520,37 @@ class Km:
         dist = np.empty(m)
         check(lib().mlb_km_predict(self._h, _ptr(pts), m, self.d, _ptr(labels), _ptr(dist)))
         return labels, dist
+
+    def transform(self, points, squared=False):
+        """Distance of every row of `points` (m, D) to every current centroid: (m, K), Euclidean or squared."""
+        pts = np.ascontiguousarray(points, dtype=np.float64)
+        assert pts.ndim == 2 and pts.shape[1] == self.d
+        m = pts.shape[0]
+        dist = np.empty((self.k, m)).T   # column-major m x K, leading dimension m
+        check(lib().mlb_km_transform(self._h, _ptr(pts), m, self.d, int(squared), _ptr(dist), max(m, 1)))
+        return dist
+
+    def transform_range(self, begin, count, squared=False):
+        """The same for the resident points [begin, begin + count) (global indices)."""
+        dist = np.empty((self.k, count)).T
+        check(lib().mlb_km_transform_range(self._h, begin, count, int(squared), _ptr(dist), max(count, 1)))
+        return dist
+
+    def score(self, points, want_sqdist=True):
+        """Inertia of the rows of `points` (m, D) under the current centroids: (squared distances or None, inertia)."""
+        pts = np.ascontiguousarray(points, dtype=np.float64)
+        assert pts.ndim == 2 and pts.shape[1] == self.d
+        m = pts.shape[0]
+        dist = np.empty(m) if want_sqdist else None
+        inertia = ctypes.c_double()
+        check(lib().mlb_km_score(self._h, _ptr(pts), m, self.d, _ptr(dist), ctypes.byref(inertia)))
+        return dist, inertia.value
+
+    def score_fitted(self):
+        """Inertia of the resident points under the current centroids (the next assign's inertia, bitwise)."""
+        inertia = ctypes.c_double()
+        check(lib().mlb_km_score_fitted(self._h, ctypes.byref(inertia)))
+        return inertia.value
 
     def get_labels(self, labels_out=None):
         labels = np.empty(self.n_local, dtype=np.uint32) if labels_out is None else labels_out

@@ -500,6 +500,78 @@ __global__ void __launch_bounds__(kKmExactTile) km_assign_exact_kernel(const KmA
     }
 }
 
+// ---------------------------------------------------------------- distances to every centroid (mlb_km_transform)
+// out[i + k ld] = (x_i - c_k).squaredNorm() as exact_distance and km_assign_exact_kernel evaluate it (the sequential
+// fused multiply-add chain over the dimensions from 0.0, raw coordinates), or its square root, for every point of the
+// tile and every centroid.  The shape of km_assign_exact_kernel: one thread per point, a 128-point tile (odd row stride)
+// and a block of centroids in shared memory; the block is stored dimension-major, so the kKmTrGroup centroids a thread
+// advances together are read as broadcast double2 loads.  A warp's stores along a column are 256 contiguous bytes.  Its
+// own argument struct: a field added to KmArgs would move the register allocation of the fit's kernels.
+constexpr int kKmTrBlock = 32;   // centroids per shared-memory block
+constexpr int kKmTrGroup = 8;    // independent distance chains per thread
+
+struct KmTransformArgs {
+    const double* x;      // n x D, point-major
+    long long n;
+    int d, k;
+    const double* craw;   // D x K
+    double* out;          // column-major n x K with leading dimension ld
+    long long ld;
+    int squared;          // 0: Euclidean distances, else squared
+};
+
+inline size_t km_transform_smem_bytes(int d)
+{
+    return sizeof(double) * (static_cast<size_t>(kKmExactTile) * (d | 1) + static_cast<size_t>(kKmTrBlock) * d);
+}
+
+__global__ void __launch_bounds__(kKmExactTile) km_transform_kernel(const KmTransformArgs p)
+{
+    extern __shared__ __align__(16) double sm[];
+    const int d = p.d, XS = d | 1, tid = threadIdx.x;
+    double* X = sm;                                            // [128][XS]
+    double* C = X + static_cast<size_t>(kKmExactTile) * XS;    // [d][32]: C[l * 32 + kk] = coordinate l of centroid c0 + kk
+    const long long tile0 = static_cast<long long>(blockIdx.x) * kKmExactTile;
+    const int nvalid = static_cast<int>(p.n - tile0 < kKmExactTile ? p.n - tile0 : kKmExactTile);
+    const FastDiv by_d(d);
+    const double* xg = p.x + tile0 * d;
+    for (int e = tid; e < nvalid * d; e += kKmExactTile) {
+        const int pt = by_d.div(e);
+        X[pt * XS + (e - pt * d)] = __ldg(xg + e);
+    }
+    const double* row = X + tid * XS;
+    double* out = p.out + tile0 + tid;
+    for (int c0 = 0; c0 < p.k; c0 += kKmTrBlock) {
+        const int cb = min(kKmTrBlock, p.k - c0);
+        __syncthreads();   // the previous block has been consumed (first pass: the tile is complete)
+        for (int e = tid; e < kKmTrBlock * d; e += kKmExactTile) {
+            const int kk = by_d.div(e), l = e - kk * d;
+            C[l * kKmTrBlock + kk] = kk < cb ? __ldg(p.craw + static_cast<long long>(c0) * d + e) : 0.0;
+        }
+        __syncthreads();
+        if (tid >= nvalid) continue;
+        for (int g0 = 0; g0 < cb; g0 += kKmTrGroup) {
+            double s[kKmTrGroup];
+#pragma unroll
+            for (int u = 0; u < kKmTrGroup; ++u) s[u] = 0.0;
+            for (int l = 0; l < d; ++l) {
+                const double xv = row[l];
+                const double2* cp = reinterpret_cast<const double2*>(C + l * kKmTrBlock + g0);
+#pragma unroll
+                for (int h = 0; h < kKmTrGroup / 2; ++h) {
+                    const double2 cv = cp[h];
+                    const double t0 = xv - cv.x, t1 = xv - cv.y;
+                    s[2 * h] = fma(t0, t0, s[2 * h]);
+                    s[2 * h + 1] = fma(t1, t1, s[2 * h + 1]);
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < kKmTrGroup; ++u)
+                if (g0 + u < cb) out[static_cast<long long>(c0 + g0 + u) * p.ld] = p.squared ? s[u] : sqrt(s[u]);
+        }
+    }
+}
+
 // ---------------------------------------------------------------- update statistics (KMeans.cpp:180-192)
 // Per chunk and cluster: the count and the sum of z = x - shift over the chunk's points carrying that label, added in
 // index order: no floating-point atomics, bitwise reproducible.  A separate kernel (it re-reads the points and the fresh
@@ -1114,6 +1186,82 @@ static int launch_assign(mlb_km* km, int g, const double* x, long long n, int ch
     return MLB_OK;
 }
 
+constexpr int64_t kKmStage = 1 << 20;   // host points per staged batch
+constexpr int kKmRun = 2048;            // chunk of the assignment kernel on host points: one inertia partial per run
+
+// The assignment of m host points with the current centroids (mlb_km_predict, mlb_km_score), on the first local GPU, in
+// staged batches of kKmStage points through the COMPACT kernels.  labels_out, sqdist_out and run_inertia (appended: the
+// inertia of every kKmRun-point run, in point order) may each be null.  The fit's labels, statistics and centroids are
+// not touched.
+static int km_assign_host(mlb_km* km, const double* x, int64_t m, int64_t ld_x, unsigned* labels_out, double* sqdist_out, std::vector<double>* run_inertia)
+{
+    Gpu& gpu = km->ctx->gpus[0];
+    const int d = km->d;
+    MLB_CUDA(cudaSetDevice(gpu.device));
+    const int64_t cap = std::min<int64_t>(m, kKmStage);
+    const int64_t cap_chunks = (cap + kKmRun - 1) / kKmRun;
+    double *xd = nullptr, *dist = nullptr, *partials = nullptr, *tmp_dist = nullptr, *tmp_scratch = nullptr;
+    unsigned *labels = nullptr, *tmp_best_lab = nullptr, *tmp_lab = nullptr;
+    std::vector<double> host_partials;
+    auto body = [&]() -> int {
+        MLB_CUDA(cudaMallocFromPoolAsync(&xd, sizeof(double) * cap * d, gpu.pool, gpu.stream));
+        MLB_CUDA(cudaMallocFromPoolAsync(&dist, sizeof(double) * cap, gpu.pool, gpu.stream));
+        MLB_CUDA(cudaMallocFromPoolAsync(&labels, sizeof(unsigned) * cap, gpu.pool, gpu.stream));
+        MLB_CUDA(cudaMallocFromPoolAsync(&partials, sizeof(double) * 8 * cap_chunks, gpu.pool, gpu.stream));
+        MLB_CUDA(cudaMemsetAsync(labels, 0, sizeof(unsigned) * cap, gpu.stream));   // the kernel reads the "previous" labels
+        if (km->nblocks > 1) {
+            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_best_lab, sizeof(unsigned) * cap, gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_lab, sizeof(unsigned) * cap, gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_dist, sizeof(double) * cap, gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_scratch, sizeof(double) * 8 * cap_chunks, gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMemsetAsync(tmp_lab, 0, sizeof(unsigned) * cap, gpu.stream));
+        }
+        for (int64_t off = 0; off < m; off += kKmStage) {
+            const int64_t n = std::min<int64_t>(kKmStage, m - off);
+            const int n_chunks = static_cast<int>((n + kKmRun - 1) / kKmRun);
+            MLB_TRY(staged_h2d(gpu, xd, x + off * ld_x, static_cast<size_t>(n), sizeof(double) * d, sizeof(double) * ld_x));
+            MLB_TRY(launch_assign(km, 0, xd, n, kKmRun, n_chunks, labels, dist, partials, 8, 0, tmp_best_lab, nullptr, tmp_lab, tmp_dist, tmp_scratch));
+            if (labels_out) MLB_TRY(staged_d2h(gpu, labels_out + off, labels, sizeof(unsigned) * n));
+            if (sqdist_out) MLB_TRY(staged_d2h(gpu, sqdist_out + off, dist, sizeof(double) * n));
+            if (run_inertia) {
+                // the stages are whole runs, so the run partials do not depend on the staging
+                host_partials.resize(static_cast<size_t>(8) * n_chunks);
+                MLB_CUDA(cudaMemcpyAsync(host_partials.data(), partials, sizeof(double) * host_partials.size(), cudaMemcpyDeviceToHost, gpu.stream));
+                MLB_CUDA(cudaStreamSynchronize(gpu.stream));
+                for (int c = 0; c < n_chunks; ++c) run_inertia->push_back(host_partials[static_cast<size_t>(8) * c]);
+            }
+            MLB_CUDA(cudaStreamSynchronize(gpu.stream));
+        }
+        return MLB_OK;
+    };
+    const int rc = body();
+    for (void* ptr : {static_cast<void*>(xd), static_cast<void*>(dist), static_cast<void*>(labels), static_cast<void*>(partials), static_cast<void*>(tmp_best_lab),
+                      static_cast<void*>(tmp_lab), static_cast<void*>(tmp_dist), static_cast<void*>(tmp_scratch)})
+        if (ptr) cudaFreeAsync(ptr, gpu.stream);
+    return rc;
+}
+
+// Points per staged batch of mlb_km_transform / mlb_km_transform_range: at most kKmStage, and at most 1 GiB of distances
+// in the device buffer (K = 256: 512K points).
+static int64_t km_transform_stage(int k)
+{
+    return std::max<int64_t>(kKmExactTile, std::min<int64_t>(kKmStage, (int64_t{1} << 27) / k / kKmExactTile * kKmExactTile));
+}
+
+// Distances of the n points at x (device memory of local GPU g) to every current centroid into out (column-major n x K,
+// leading dimension ld).
+static int launch_transform(mlb_km* km, int g, const double* x, long long n, int squared, double* out, long long ld)
+{
+    Gpu& gpu = km->ctx->gpus[g];
+    const KmTransformArgs a{x, n, km->d, km->k, km->gpus[g].craw, out, ld, squared};
+    const size_t smem = km_transform_smem_bytes(km->d);
+    MLB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(km_transform_kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    km_transform_kernel<<<static_cast<unsigned>((n + kKmExactTile - 1) / kKmExactTile), kKmExactTile, smem, gpu.stream>>>(a);
+    MLB_CUDA(cudaGetLastError());
+    ++km->launches;
+    return MLB_OK;
+}
+
 }  // namespace mlb
 
 extern "C" {
@@ -1341,43 +1489,154 @@ int mlb_km_predict(mlb_km* km, const double* x, int64_t m, int64_t ld_x, unsigne
     MLB_REQUIRE(m >= 0 && ld_x >= km->d, "mlb_km_predict: bad shape (m=%lld, ld_x=%lld, D=%d)", static_cast<long long>(m), static_cast<long long>(ld_x), km->d);
     if (!km->have_centroids) { set_error("mlb_km_predict: centroids not set"); return MLB_ESTATE; }
     if (m == 0) return MLB_OK;
-    constexpr int64_t kStage = 1 << 20;   // points per staged batch
-    constexpr int kChunk = 2048;          // the assignment kernel leaves one (unused here) inertia partial per chunk
+    return km_assign_host(km, x, m, ld_x, labels_out, sqdist_out, nullptr);
+}
+
+int mlb_km_score(mlb_km* km, const double* x, int64_t m, int64_t ld_x, double* sqdist_out, double* inertia_out)
+{
+    MLB_ENTER(km ? km->ctx : nullptr);
+    MLB_REQUIRE(km && x && inertia_out, "mlb_km_score: null argument");
+    MLB_REQUIRE(m >= 0 && ld_x >= km->d, "mlb_km_score: bad shape (m=%lld, ld_x=%lld, D=%d)", static_cast<long long>(m), static_cast<long long>(ld_x), km->d);
+    if (!km->have_centroids) { set_error("mlb_km_score: centroids not set"); return MLB_ESTATE; }
+    *inertia_out = 0.0;
+    if (m == 0) return MLB_OK;
+    std::vector<double> runs;
+    MLB_TRY(km_assign_host(km, x, m, ld_x, nullptr, sqdist_out, &runs));
+    double total = 0.0;
+    for (double v : runs) total += v;   // in point order
+    *inertia_out = total;
+    return MLB_OK;
+}
+
+int mlb_km_score_fitted(mlb_km* km, double* inertia_out)
+{
+    MLB_ENTER(km ? km->ctx : nullptr);
+    MLB_REQUIRE(km && inertia_out, "mlb_km_score_fitted: null argument");
+    if (!km->have_centroids) { set_error("mlb_km_score_fitted: centroids not set"); return MLB_ESTATE; }
+    mlb_ctx* ctx = km->ctx;
+    const size_t ng = ctx->gpus.size();
+    // The assignment of mlb_km_assign (same kernels, same chunks) into scratch labels and 8 scalars per chunk; the chunk
+    // inertias take the step's reduction (8 virtual shards, one exchange, fixed tree), so the sum is bitwise the inertia
+    // the next mlb_km_assign reports, for any GPU count.  The fit's labels, statistics, centroids and timer are not touched;
+    // the temporaries of the centroid-block path are rewritten by every assignment before they are read.
+    std::vector<unsigned*> labels(ng, nullptr);
+    std::vector<double*> part(ng, nullptr), vsum(ng, nullptr);
+    ReduceScratch scratch;
+    double host_vsum[kVirtualShards * 8] = {};
+    auto body = [&]() -> int {
+        MLB_TRY(for_each_gpu(ctx, [&](int g, Gpu& gpu) -> int {
+            KmGpu& kg = km->gpus[g];
+            const DataShard& sh = km->data->shards[g];
+            const int n_chunks = static_cast<int>(sh.n_chunks());
+            MLB_CUDA(cudaMallocFromPoolAsync(&labels[g], sizeof(unsigned) * std::max<int64_t>(1, sh.n()), gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMallocFromPoolAsync(&part[g], sizeof(double) * 8 * std::max(1, n_chunks), gpu.pool, gpu.stream));
+            MLB_CUDA(cudaMallocFromPoolAsync(&vsum[g], sizeof(double) * kVirtualShards * 8, gpu.pool, gpu.stream));
+            if (n_chunks > 0)
+                MLB_TRY(launch_assign(km, g, sh.x, sh.n(), km->data->lay.chunk, n_chunks, labels[g], nullptr, part[g], 8, 0, kg.best_lab, kg.best_dist, kg.lab_tmp,
+                                      kg.dist_tmp, kg.scratch));
+            return MLB_OK;
+        }));
+        MLB_TRY(reduce_and_exchange(km->data, part, vsum, 8, scratch));
+        km->launches += static_cast<int64_t>(ng);
+        Gpu& gpu0 = ctx->gpus[0];
+        MLB_CUDA(cudaSetDevice(gpu0.device));
+        MLB_CUDA(cudaMemcpyAsync(host_vsum, vsum[0], sizeof(host_vsum), cudaMemcpyDeviceToHost, gpu0.stream));
+        return MLB_OK;
+    };
+    int rc = body();
+    const int rc_sync = mlb_ctx_synchronize(ctx);
+    if (rc == MLB_OK) rc = rc_sync;
+    for (size_t g = 0; g < ng; ++g) {
+        cudaSetDevice(ctx->gpus[g].device);
+        for (void* ptr : {static_cast<void*>(labels[g]), static_cast<void*>(part[g]), static_cast<void*>(vsum[g])})
+            if (ptr) cudaFreeAsync(ptr, ctx->gpus[g].stream);
+    }
+    scratch.release(ctx);
+    if (rc == MLB_OK) *inertia_out = tree8(host_vsum, 8);
+    return rc;
+}
+
+int mlb_km_transform(mlb_km* km, const double* x, int64_t m, int64_t ld_x, int squared, double* dist_out, int64_t ld_out)
+{
+    MLB_ENTER(km ? km->ctx : nullptr);
+    MLB_REQUIRE(km && x && dist_out, "mlb_km_transform: null argument");
+    MLB_REQUIRE(m >= 0 && ld_x >= km->d && ld_out >= m, "mlb_km_transform: bad shape (m=%lld, ld_x=%lld, ld_out=%lld, D=%d)", static_cast<long long>(m),
+                static_cast<long long>(ld_x), static_cast<long long>(ld_out), km->d);
+    if (!km->have_centroids) { set_error("mlb_km_transform: centroids not set"); return MLB_ESTATE; }
+    if (m == 0) return MLB_OK;
     Gpu& gpu = km->ctx->gpus[0];
     const int d = km->d;
     MLB_CUDA(cudaSetDevice(gpu.device));
-    const int64_t cap = std::min<int64_t>(m, kStage);
-    const int64_t cap_chunks = (cap + kChunk - 1) / kChunk;
-    double *xd = nullptr, *dist = nullptr, *partials = nullptr, *tmp_dist = nullptr, *tmp_scratch = nullptr;
-    unsigned *labels = nullptr, *tmp_best_lab = nullptr, *tmp_lab = nullptr;
+    const int64_t stage = km_transform_stage(km->k), cap = std::min(m, stage);
+    double *xd = nullptr, *out = nullptr;
     auto body = [&]() -> int {
         MLB_CUDA(cudaMallocFromPoolAsync(&xd, sizeof(double) * cap * d, gpu.pool, gpu.stream));
-        MLB_CUDA(cudaMallocFromPoolAsync(&dist, sizeof(double) * cap, gpu.pool, gpu.stream));
-        MLB_CUDA(cudaMallocFromPoolAsync(&labels, sizeof(unsigned) * cap, gpu.pool, gpu.stream));
-        MLB_CUDA(cudaMallocFromPoolAsync(&partials, sizeof(double) * 8 * cap_chunks, gpu.pool, gpu.stream));
-        MLB_CUDA(cudaMemsetAsync(labels, 0, sizeof(unsigned) * cap, gpu.stream));   // the kernel reads the "previous" labels
-        if (km->nblocks > 1) {
-            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_best_lab, sizeof(unsigned) * cap, gpu.pool, gpu.stream));
-            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_lab, sizeof(unsigned) * cap, gpu.pool, gpu.stream));
-            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_dist, sizeof(double) * cap, gpu.pool, gpu.stream));
-            MLB_CUDA(cudaMallocFromPoolAsync(&tmp_scratch, sizeof(double) * 8 * cap_chunks, gpu.pool, gpu.stream));
-            MLB_CUDA(cudaMemsetAsync(tmp_lab, 0, sizeof(unsigned) * cap, gpu.stream));
-        }
-        for (int64_t off = 0; off < m; off += kStage) {
-            const int64_t n = std::min<int64_t>(kStage, m - off);
+        MLB_CUDA(cudaMallocFromPoolAsync(&out, sizeof(double) * cap * km->k, gpu.pool, gpu.stream));
+        for (int64_t off = 0; off < m; off += stage) {
+            const int64_t n = std::min(stage, m - off);
             MLB_TRY(staged_h2d(gpu, xd, x + off * ld_x, static_cast<size_t>(n), sizeof(double) * d, sizeof(double) * ld_x));
-            MLB_TRY(launch_assign(km, 0, xd, n, kChunk, static_cast<int>((n + kChunk - 1) / kChunk), labels, dist, partials, 8, 0,
-                                  tmp_best_lab, nullptr, tmp_lab, tmp_dist, tmp_scratch));
-            MLB_TRY(staged_d2h(gpu, labels_out + off, labels, sizeof(unsigned) * n));
-            if (sqdist_out) MLB_TRY(staged_d2h(gpu, sqdist_out + off, dist, sizeof(double) * n));
+            MLB_TRY(launch_transform(km, 0, xd, n, squared, out, cap));
+            MLB_TRY(staged_d2h_2d(gpu, dist_out + off, sizeof(double) * ld_out, out, sizeof(double) * cap, static_cast<size_t>(km->k), sizeof(double) * n));
             MLB_CUDA(cudaStreamSynchronize(gpu.stream));
         }
         return MLB_OK;
     };
     const int rc = body();
-    for (void* ptr : {static_cast<void*>(xd), static_cast<void*>(dist), static_cast<void*>(labels), static_cast<void*>(partials), static_cast<void*>(tmp_best_lab),
-                      static_cast<void*>(tmp_lab), static_cast<void*>(tmp_dist), static_cast<void*>(tmp_scratch)})
+    for (double* ptr : {xd, out})
         if (ptr) cudaFreeAsync(ptr, gpu.stream);
+    return rc;
+}
+
+int mlb_km_transform_range(mlb_km* km, int64_t begin, int64_t count, int squared, double* dist_out, int64_t ld_out)
+{
+    MLB_ENTER(km ? km->ctx : nullptr);
+    MLB_REQUIRE(km && dist_out, "mlb_km_transform_range: null argument");
+    MLB_REQUIRE(begin >= 0 && count >= 0 && begin + count <= km->data->lay.n_total, "mlb_km_transform_range: range out of bounds");
+    MLB_REQUIRE(ld_out >= count, "mlb_km_transform_range: leading dimension smaller than the row count");
+    if (!km->have_centroids) { set_error("mlb_km_transform_range: centroids not set"); return MLB_ESTATE; }
+    if (count == 0) return MLB_OK;
+    mlb_ctx* ctx = km->ctx;
+    const size_t ng = ctx->gpus.size();
+    std::vector<int64_t> cap(ng, 0);
+    int64_t covered = 0;
+    const int64_t stage = km_transform_stage(km->k);
+    for (size_t g = 0; g < ng; ++g) {
+        const DataShard& sh = km->data->shards[g];
+        const int64_t held = std::max<int64_t>(0, std::min(begin + count, sh.end) - std::max(begin, sh.begin));
+        covered += held;
+        cap[g] = std::min(held, stage);
+    }
+    MLB_REQUIRE(covered == count, "mlb_km_transform_range: range is not held by this context");
+    std::vector<double*> out(ng, nullptr);
+    auto body = [&]() -> int {
+        MLB_TRY(for_each_gpu(ctx, [&](int g, Gpu& gpu) -> int {
+            if (cap[g] > 0) MLB_CUDA(cudaMallocFromPoolAsync(&out[g], sizeof(double) * cap[g] * km->k, gpu.pool, gpu.stream));
+            return MLB_OK;
+        }));
+        // stage by stage: up to `stage` points per GPU at a time through its device buffer
+        for (int64_t off = 0;; off += stage) {
+            bool any = false;
+            MLB_TRY(for_each_gpu(ctx, [&](int g, Gpu& gpu) -> int {
+                const DataShard& sh = km->data->shards[g];
+                const int64_t lo = std::max(begin, sh.begin) + off, hi = std::min(begin + count, sh.end);
+                const int64_t n = std::min(stage, hi - lo);
+                if (n <= 0) return MLB_OK;
+                any = true;
+                MLB_TRY(launch_transform(km, g, sh.x + (lo - sh.begin) * km->d, n, squared, out[g], cap[g]));
+                return staged_d2h_2d(gpu, dist_out + (lo - begin), sizeof(double) * ld_out, out[g], sizeof(double) * cap[g], static_cast<size_t>(km->k), sizeof(double) * n);
+            }));
+            if (!any) break;
+        }
+        return MLB_OK;
+    };
+    int rc = body();
+    const int rc_sync = mlb_ctx_synchronize(ctx);
+    if (rc == MLB_OK) rc = rc_sync;
+    for (size_t g = 0; g < ng; ++g)
+        if (out[g]) {
+            cudaSetDevice(ctx->gpus[g].device);
+            cudaFreeAsync(out[g], ctx->gpus[g].stream);
+        }
     return rc;
 }
 

@@ -1,7 +1,9 @@
 #pragma once
 // ml::Clustering::KMeans: Lloyd's algorithm with the reference's public surface
-// (ML/KMeans.hpp:19-101) on the B200 backend.  Additions: number_iterations(), and assign_labels(points), the
-// batched form of assign_label(x) on the device.
+// (ML/KMeans.hpp:19-101) on the B200 backend.  Additions: number_iterations(); assign_labels(points), the
+// batched form of assign_label(x) on the device; transform(points) and transform(), the distance of every point to
+// every centroid, and inertia(points) and final_inertia(), the inertia at the returned centroids, for new points or the
+// fitted ones, on the device.
 #include "Clustering.hpp"
 #include <memory>
 #include <vector>
@@ -59,8 +61,31 @@ namespace ml
             @throw std::logic_error If there is no fitted device state (no fit yet, or the N == K exact fit). */
             DLL_DECLSPEC std::pair<std::vector<unsigned int>, std::vector<double>> assign_labels(DataView points) const;
 
-            /** Sum of squared distances of the points to their centroids. */
+            /** Sum of squared distances of the points to their centroids, from the last assignment of the fit (when the fit
+            stops at maximum_steps, that assignment came before the last update: see final_inertia()). */
             double inertia() const { return inertia_; }
+
+            /** Euclidean distance of every column of `points` (D x m) to every centroid, m x K, on the device.
+            @throw std::invalid_argument If `points` has the wrong number of rows.
+            @throw std::logic_error If there is no fitted device state (no fit yet, the N == K exact fit, or after
+            release_device()). */
+            DLL_DECLSPEC Eigen::MatrixXd transform(DataView points) const;
+
+            /** The same for the fitted points (this process's own points under ml::Distributed): N x K, N K 8 bytes of host
+            memory (205 GB at N = 1e8, K = 256; the cppyml binding copies the result into its numpy array, so through Python
+            the peak is twice that).
+            @throw std::logic_error If there is no fitted device state. */
+            DLL_DECLSPEC Eigen::MatrixXd transform() const;
+
+            /** Sum over the columns of `points` of the squared distance to the nearest centroid, on the device.
+            @throw std::invalid_argument If `points` has the wrong number of rows.
+            @throw std::logic_error If there is no fitted device state. */
+            DLL_DECLSPEC double inertia(DataView points) const;
+
+            /** The inertia of the fitted points at the centroids the fit returned: inertia() whenever the fit ended on an
+            assignment to those centroids.  Under ml::Distributed: over all ranks' points, and collective.
+            @throw std::logic_error If there is no fitted device state. */
+            DLL_DECLSPEC double final_inertia() const;
 
             bool converged() const override { return converged_; }
 

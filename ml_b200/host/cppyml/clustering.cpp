@@ -204,6 +204,34 @@ namespace ml
 				std::memcpy(distances.mutable_data(), result.second.data(), sizeof(double) * result.second.size());
 				return std::make_pair(labels, distances);
 			}
+
+			/** Euclidean distance of every row of `data` (m, D), or of every fitted point when `data` is None, to every
+			centroid: (m, K), on the device. */
+			py::array_t<double> transform_py(const py::object& data) const
+			{
+				Eigen::MatrixXd result;
+				if (data.is_none()) {
+					py::gil_scoped_release release;
+					result = transform();
+				} else {
+					const auto columns = as_columns(data);
+					py::gil_scoped_release release;
+					result = transform(columns);
+				}
+				return to_numpy(result);
+			}
+
+			/** -inertia of the rows of `data`, or of the fitted points at the returned centroids when `data` is None. */
+			double score_py(const py::object& data) const
+			{
+				if (data.is_none()) {
+					py::gil_scoped_release release;
+					return -final_inertia();
+				}
+				const auto columns = as_columns(data);
+				py::gil_scoped_release release;
+				return -inertia(columns);
+			}
 		};
 	}
 }
@@ -303,7 +331,7 @@ void init_clustering(py::module_& m)
 		.def_property_readonly("centroids", &ml::Clustering::KMeansPy::centroids_row_major, "Centroids after the fit, shape (K, D).")
 		.def_property_readonly("labels", &ml::Clustering::KMeansPy::labels, "Cluster index of every fitted point (a list, as in the reference; brought to the host on first access).")
 		.def_property_readonly("labels_array", [](const ml::Clustering::KMeansPy& km) { return to_numpy(km.labels()); }, "The same as a uint32 numpy array (an addition: a Python list of 1e8 integers takes gigabytes).")
-		.def_property_readonly("inertia", &ml::Clustering::KMeansPy::inertia, "Sum of the squared distances of the points to their centroids.")
+		.def_property_readonly("inertia", [](const ml::Clustering::KMeansPy& km) { return km.inertia(); }, "Sum of the squared distances of the points to their centroids.")
 		.def_property_readonly("converged", &ml::Clustering::KMeansPy::converged, "Whether the last fit converged.")
 		.def_property_readonly("number_iterations", &ml::Clustering::KMeansPy::number_iterations, "Assignment steps run by the last fit.")
 		.def("assign_label", &ml::Clustering::KMeansPy::assign_label_py, py::arg("x"),
@@ -311,6 +339,10 @@ void init_clustering(py::module_& m)
 		.def("release_device", &ml::Clustering::KMeansPy::release_device, py::arg("keep_results") = true, "Frees the GPU memory the last fit still holds; with keep_results the labels are brought to the host first.")
 		.def("assign_labels", &ml::Clustering::KMeansPy::assign_labels_py, py::arg("data").noconvert(),
 			"Assigns every row of data to its closest cluster (computed on the GPU).\n\nArgs:\n    data: A 2D float64 C-contiguous array with data points in rows.\n\nReturns:\n    Tuple of the array of cluster labels and the array of squared Euclidean distances to the cluster centroids.")
+		.def("transform", &ml::Clustering::KMeansPy::transform_py, py::arg("data").noconvert() = py::none(),
+			"Euclidean distance of every point to every centroid (computed on the GPU), as sklearn's KMeans.transform.\n\nArgs:\n    data: A 2D float64 C-contiguous array of shape (m, D) with points in rows, or None for the fitted points (still on the GPU).\n\nReturns:\n    Array of shape (m, K).  For the fitted points that is N K 8 bytes, and the call briefly holds twice that in host memory (the result is copied into the array).")
+		.def("score", &ml::Clustering::KMeansPy::score_py, py::arg("data").noconvert() = py::none(),
+			"Opposite of the inertia, the sum of the squared distances of the points to their nearest centroids (computed on the GPU), as sklearn's KMeans.score.  With data=None it is the inertia of the fitted points at the centroids the fit returned (the inertia property belongs to the last assignment of the fit, which precedes the last update when the fit stops at maximum_steps).\n\nArgs:\n    data: A 2D float64 C-contiguous array of shape (m, D), or None for the fitted points.")
 		.doc() = "Lloyd's K-means on B200 GPUs.";
 
 	m.def("_standardise_features", [](const py::array& features) {

@@ -84,6 +84,11 @@ namespace ml
 			if (distributed_active) {
 				// one process per GPU: `data` holds this rank's columns, the problem is the concatenation over the ranks
 				check(mlb_ctx_sum_int64(ctx, data.cols(), &total), "point count over the ranks");
+				int world = 0, n_local = 0, rank = 0;
+				int64_t begin = 0, end = 0;
+				check(mlb_ctx_world(ctx, &world, &n_local, &rank), "world");
+				check(mlb_shard_range(total, world, rank, &begin, &end), "shard range");
+				begin_ = begin;
 			}
 			check(mlb_data_upload(ctx, data.data(), data.cols(), total, static_cast<int>(data.rows()), data.outerStride(), &handle_), "upload");
 		}
@@ -240,7 +245,7 @@ namespace ml
 		}
 
 		KmDevice::KmDevice(std::shared_ptr<DeviceData> data, unsigned int number_clusters)
-			: data_(std::move(data))
+			: data_(std::move(data)), number_clusters_(number_clusters)
 		{
 			check(mlb_km_create(shared_context(), data_->handle(), static_cast<int>(number_clusters), &km_), "KMeans");
 		}
@@ -281,6 +286,38 @@ namespace ml
 			labels.resize(static_cast<size_t>(points.cols()));
 			squared_distances.resize(static_cast<size_t>(points.cols()));
 			check(mlb_km_predict(km_, points.data(), points.cols(), points.outerStride(), labels.data(), squared_distances.data()), "KMeans labels of new points");
+		}
+
+		void KmDevice::transform(Eigen::Ref<const Eigen::MatrixXd> points, Eigen::MatrixXd& distances)
+		{
+			distances.resize(points.cols(), number_clusters_);
+			if (!points.cols()) {
+				return;
+			}
+			check(mlb_km_transform(km_, points.data(), points.cols(), points.outerStride(), 0, distances.data(), std::max<Eigen::Index>(1, points.cols())), "KMeans distances of new points");
+		}
+
+		void KmDevice::transform_fitted(Eigen::MatrixXd& distances)
+		{
+			distances.resize(data_->cols(), number_clusters_);
+			check(mlb_km_transform_range(km_, data_->begin(), data_->cols(), 0, distances.data(), std::max<Eigen::Index>(1, data_->cols())), "KMeans distances of the fitted points");
+		}
+
+		double KmDevice::inertia(Eigen::Ref<const Eigen::MatrixXd> points)
+		{
+			double inertia = 0;
+			if (!points.cols()) {
+				return inertia;
+			}
+			check(mlb_km_score(km_, points.data(), points.cols(), points.outerStride(), nullptr, &inertia), "KMeans inertia of new points");
+			return inertia;
+		}
+
+		double KmDevice::fitted_inertia()
+		{
+			double inertia = 0;
+			check(mlb_km_score_fitted(km_, &inertia), "KMeans inertia of the fitted points");
+			return inertia;
 		}
 
 		void KmDevice::get_labels(std::vector<unsigned int>& labels)

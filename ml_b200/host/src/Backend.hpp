@@ -39,12 +39,14 @@ namespace ml
 			mlb_data* handle() const { return handle_; }
 			Eigen::Index rows() const { return rows_; }
 			Eigen::Index cols() const { return cols_; }
+			/** Global index of this process's first point (0 unless under ml::Distributed). */
+			Eigen::Index begin() const { return begin_; }
 			/** KPP distance pass for the newest centroid (D doubles); `nearest` (N) receives the squared distance of
 			every point to the nearest centroid chosen so far. */
 			void kpp_update(const double* centroid, bool first, std::vector<double>& nearest);
 		private:
 			mlb_data* handle_ = nullptr;
-			Eigen::Index rows_ = 0, cols_ = 0;
+			Eigen::Index rows_ = 0, cols_ = 0, begin_ = 0;
 		};
 
 		/** What `std::discrete_distribution<Eigen::Index>(weights.begin(), weights.end())(prng)` returns and consumes
@@ -108,10 +110,19 @@ namespace ml
 			void get_labels(std::vector<unsigned int>& labels);
 			/** Nearest centroid and squared distance for every column of `points` (D x m). */
 			void predict(Eigen::Ref<const Eigen::MatrixXd> points, std::vector<unsigned int>& labels, std::vector<double>& squared_distances);
+			/** Euclidean distance of every column of `points` (D x m) to every current centroid: m x K. */
+			void transform(Eigen::Ref<const Eigen::MatrixXd> points, Eigen::MatrixXd& distances);
+			/** The same for the fitted points (this process's own points under ml::Distributed). */
+			void transform_fitted(Eigen::MatrixXd& distances);
+			/** Sum over the columns of `points` of the squared distance to the nearest current centroid. */
+			double inertia(Eigen::Ref<const Eigen::MatrixXd> points);
+			/** The same for all fitted points: the inertia the next assign() would return (collective under ml::Distributed). */
+			double fitted_inertia();
 			const std::shared_ptr<DeviceData>& data() const { return data_; }
 		private:
 			std::shared_ptr<DeviceData> data_;
 			mlb_km* km_ = nullptr;
+			unsigned int number_clusters_;
 		};
 
 		/** Up to four starts of a multi-start K-means fit advanced in lockstep on one resident copy of the points

@@ -234,6 +234,7 @@ namespace ml
 				labels_on_host_ = false;   // downloaded on first access to labels()
 			} else {
 				labels_on_host_ = true;    // no start converged: the last start's labels, already here
+				device.set_centroids(centroids_);   // what transform() and final_inertia() read: the returned centroids
 			}
 			return converged_;
 		}
@@ -323,6 +324,48 @@ namespace ml
 			std::pair<std::vector<unsigned int>, std::vector<double>> result;
 			device_->predict(points, result.first, result.second);
 			return result;
+		}
+
+		Eigen::MatrixXd KMeans::transform(DataView points) const
+		{
+			if (points.rows() != centroids_.rows()) {
+				throw std::invalid_argument("KMeans: wrong number of rows");
+			}
+			if (!device_) {
+				throw std::logic_error("KMeans: no fitted device state");
+			}
+			Eigen::MatrixXd result;
+			device_->transform(points, result);
+			return result;
+		}
+
+		Eigen::MatrixXd KMeans::transform() const
+		{
+			if (!device_) {
+				throw std::logic_error("KMeans: no fitted device state");
+			}
+			Eigen::MatrixXd result;
+			device_->transform_fitted(result);
+			return result;
+		}
+
+		double KMeans::inertia(DataView points) const
+		{
+			if (points.rows() != centroids_.rows()) {
+				throw std::invalid_argument("KMeans: wrong number of rows");
+			}
+			if (!device_) {
+				throw std::logic_error("KMeans: no fitted device state");
+			}
+			return device_->inertia(points);
+		}
+
+		double KMeans::final_inertia() const
+		{
+			if (!device_) {
+				throw std::logic_error("KMeans: no fitted device state");
+			}
+			return device_->fitted_inertia();
 		}
 
 		std::pair<unsigned int, double> KMeans::assign_label(PointView x) const
